@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path (rank 0 only)
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR  # + the last timed step's detections as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic input: the FAM/ODM head (conv towers, AlignConv,
 ORConv2d + RotationInvariantPooling -- every layer a kernel of this library) over the five FPN levels of `--batch`
@@ -282,6 +283,36 @@ def cuda_time(torch, fn, reps, warm=3):
     return a.elapsed_time(b) / reps
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, dets, labels, counts, odm_cls_bias):
+    """Write what one step returned to its caller as path/<name>.npy, so that two builds run with the same arguments
+    (hence the same seeded inputs) can be compared output for output: dets [n,K,6] and labels [n,K] float32, counts [n]
+    float64, rows at or past an image's count zeroed (the NMS leaves them unspecified).  n is every image of the step,
+    or a fixed seeded sample of them where all would exceed DUMP_MAX_BYTES; image_index [n] float64 names them.
+    odm_cls_bias [C] float64 is the classification bias the step ran with: calibrate_scores sets it from this build's
+    own forward pass, so outputs of two builds are comparable as they stand only where their biases are equal."""
+    import numpy as np
+    bias = odm_cls_bias.detach().double().cpu().numpy()
+    dets, labels = dets.float().cpu().numpy(), labels.float().cpu().numpy()
+    counts = counts.cpu().numpy().astype(np.float64)
+    n, K = labels.shape
+    keep = np.arange(n)
+    per_image = dets[0].nbytes + labels[0].nbytes + 16
+    budget = DUMP_MAX_BYTES - bias.nbytes
+    if n * per_image > budget:
+        keep = np.sort(np.random.default_rng(0).choice(n, budget // per_image, replace=False))
+    dets, labels, counts = dets[keep], labels[keep], counts[keep]
+    unused = np.arange(K)[None, :] >= counts[:, None]
+    dets[unused] = 0
+    labels[unused] = 0
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("dets", dets), ("labels", labels), ("counts", counts), ("image_index", keep.astype(np.float64)),
+                    ("odm_cls_bias", bias)):
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -296,7 +327,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra bench legs (configs 1-3, NMS sizes, 10k candidates)")
     ap.add_argument("--no-graph", action="store_true", help="launch eagerly instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the detections of the last timed step to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -435,6 +472,8 @@ def main():
     ms, out = timed_steps(args.steps)
     launches = _lib.launches - l0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:              # before the legs below replay the graphs into the same buffers
+        dump_outputs(args.dump_outputs, *out, head.odm_cls_head.bias)
     value = world * B * args.steps / (ms / 1e3)
     own = slice(rank * B, (rank + 1) * B) if world > 1 else slice(0, B)
     ndet = int(out[2][own].float().mean().item())

@@ -291,6 +291,16 @@ S2A_EXPORT int s2a_conv2d_forward_tc_multi2(int nlevels, int split, const void* 
                                             const float* bias0, const float* bias1, void* const* outs,
                                             const int* Hs, const int* Ws, int B, int C, int Co_pad, int ks,
                                             int relu, int dtype, void* stream);
+/* The FAM regression head -- a 1x1 conv with 5 output channels padded to Co_pad = 32 (packed by
+ * s2a_conv2d_pack_weight), + bias, no ReLU -- with the anchor decode of s2a_fam_decode in its epilogue:
+ * refined[l] [B, H_l, W_l, 5] fp32 is bit-identical to s2a_fam_decode(strides, anchor_scale, anchor_angle,
+ * wh_ratio_clip) of the head's stored output, which is never written.  One launch for all levels. */
+S2A_EXPORT int s2a_conv2d_forward_tc_fam_decode(int nlevels, const void* const* xs,
+                                                const void* packed_weight, const float* bias,
+                                                float* const* refined, const int* Hs, const int* Ws,
+                                                const float* strides, int B, int C, int Co_pad,
+                                                float anchor_scale, float anchor_angle,
+                                                double wh_ratio_clip, int dtype, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Box decode stages of the head (SURVEY.md 8(f) rows 2-3), batched over all FPN levels and images:

@@ -51,6 +51,8 @@ PROTOTYPES = {
     "s2a_conv2d_pack_weight": (_i32, [_vp, _i32, _vp, _i32, _i32, _i32, _i32, _vp]),
     "s2a_conv2d_forward_tc_multi": (_i32, [_i32, _vp, _vp, _vp, _vp, _vp, _vp] + [_i32] * 6 + [_vp]),
     "s2a_conv2d_forward_tc_multi2": (_i32, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp] + [_i32] * 6 + [_vp]),
+    "s2a_conv2d_forward_tc_fam_decode": (_i32, [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp] + [_i32] * 3 +
+                                         [_f32, _f32, _f64, _i32, _vp]),
     "s2a_deform_im2col_f32": (_i32, [_vp, _vp, _vp] + [_i32] * 13 + [_vp]),
     "s2a_deform_col2im_f32": (_i32, [_vp, _vp, _vp, _vp, _vp] + [_i32] * 13 + [_vp]),
     "s2a_assign_labels_workspace_bytes": (_sz, [_i64, _i64, _i64]),
@@ -89,7 +91,8 @@ KERNELS_PER_CALL = {
     "arf_forward": 1, "arf_backward": 1, "ri_pool": 1, "deform_conv_forward_cuda": 1, "alignconv_forward": 1,
     "orconv_forward": 1, "conv_pack_weight": 1, "alignconv_forward_tc": 1, "orconv_forward_tc": 1, "deform_conv_forward_tc": 1, "deform_conv_dgrad_tc": 9, "deform_conv_wgrad_tc": 1, "conv_pack_weight_tf32": 1, "conv_forward_tf32x3": 1,
     "alignconv_forward_tc_multi": 1, "orconv_forward_tc_multi": 1, "fam_decode": 1, "select_decode": 3, "conv2d_pack_weight": 1,
-    "conv2d_forward_tc_multi": 1, "conv2d_forward_tc_multi2": 1, "assign_labels": 2, "deform_im2col": 1, "deform_col2im": 1,
+    "conv2d_forward_tc_multi": 1, "conv2d_forward_tc_multi2": 1, "conv2d_forward_tc_fam_decode": 1,
+    "assign_labels": 2, "deform_im2col": 1, "deform_col2im": 1,
     "poly_nms": 4, "poly_iou_pairs": 1,
 }
 launches = 0          # running count, read by bench.py for "gpu_launches"

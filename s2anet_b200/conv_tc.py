@@ -398,6 +398,38 @@ def conv2d_forward_tc_multi(xs, weight, bias=None, relu=False):
     return outs if Co == Co_pad else [o[:, :Co] for o in outs]
 
 
+def conv2d_forward_tc_fam_decode(xs, head, strides, anchor_scale, anchor_angle, wh_ratio_clip=1e-6):
+    """decode.fam_decode(conv2d_forward_tc_multi(xs, head.weight, head.bias), strides, ...) in ONE launch, bit for bit,
+    without writing the deltas: the FAM regression head (nn.Conv2d(C, 5, 1) with bias) decodes its output against the
+    grid anchors in its epilogue.  xs[l] [B,C,H_l,W_l] bf16/fp16 -> refined anchors [B,H_l,W_l,5] fp32 per level."""
+    w, b = head.weight, head.bias
+    if w.dim() != 4 or tuple(w.shape[0:1]) + tuple(w.shape[2:]) != (5, 1, 1) or b is None:
+        raise ValueError("conv2d_forward_tc_fam_decode: needs a 5-channel 1x1 head with bias")
+    if tuple(head.stride) != (1, 1) or tuple(head.padding) != (0, 0) or tuple(head.dilation) != (1, 1) or head.groups != 1:
+        raise ValueError("conv2d_forward_tc_fam_decode: the head must have stride 1, no padding, dilation 1, one group")
+    if len(strides) != len(xs):
+        raise ValueError("conv2d_forward_tc_fam_decode: one anchor stride per level")
+    B, C = xs[0].shape[:2]
+    if any(x.dim() != 4 or x.size(1) != w.size(1) for x in xs):
+        raise ValueError("conv2d_forward_tc_fam_decode: inputs must be [B,%d,H,W]" % w.size(1))
+    if C % 8:
+        raise ValueError("conv2d_forward_tc_fam_decode: C must be a multiple of 8")
+    dev = _lib.require_cuda(*xs, w, b)
+    packed, bp, Co_pad, _ = pack_conv2d_weight(w, b, xs[0].dtype)
+    xc = [_nhwc(x) for x in xs]
+    refined = [torch.empty((B, x.size(2), x.size(3), 5), dtype=torch.float32, device=dev) for x in xs]
+    import ctypes as C_
+    st = (C_.c_float * len(xs))(*[float(s) for s in strides])
+    with torch.cuda.device(dev):
+        rc = _lib.load().s2a_conv2d_forward_tc_fam_decode(len(xs), _ptr_array(xc), _lib.ptr(packed), _lib.ptr(bp),
+                                                          _ptr_array(refined), _int_array([x.size(2) for x in xs]),
+                                                          _int_array([x.size(3) for x in xs]), st, B, C, Co_pad,
+                                                          float(anchor_scale), float(anchor_angle), float(wh_ratio_clip),
+                                                          _lib.dtype_code(xc[0]), _lib.stream_ptr(dev))
+    _lib.check(rc, "conv2d_forward_tc_fam_decode")
+    return refined
+
+
 def conv2d_forward_tc_pair(xs0, weight0, bias0, xs1, weight1, bias1, relu=False):
     """Two convolutions of one shape class -- same C, padded C_out, kernel size, ReLU and batch, e.g. the
     classification and the regression tower layer of the head -- in ONE persistent launch (two launches of 682 tile

@@ -36,6 +36,7 @@
 #include <cstring>
 #include <type_traits>
 
+#include "box_decode.cuh"
 #include "common.cuh"
 
 namespace s2a {
@@ -132,6 +133,7 @@ struct TcLevel {
   int H, W, tiles_x, tiles_y;
   int tile_begin;         // first global tile index of this level
   float stride;
+  float* refine;          // FAM decode (conv_tc_kernel<TC_PLAIN, T, true>): [B, H, W, 5] fp32 refined anchors
 };
 
 struct TcParams {
@@ -160,6 +162,10 @@ struct TcParams {
   const void* sc_off;     // [B, 18, H, W] offsets, fp32 or the 16-bit type
   int sc_off_f32;
   int sc_tap;             // -1: ordinary epilogue
+  // TC_PLAIN, 1 x 1, FAM-decode epilogue (conv_tc_kernel<TC_PLAIN, T, true>): the first 5 output channels are the FAM
+  // regression deltas; they are rounded to T exactly as the ordinary epilogue stores them and decoded against the grid
+  // anchor (models/head.py:27-52) instead of being stored.
+  float fd_scale, fd_angle, fd_lim;   // anchor scale, anchor angle, dw / dh clamp bound (rounded to T)
 };
 
 struct TileCoord { int lvl, b, ty0, tx0; };
@@ -601,9 +607,10 @@ __device__ __forceinline__ void build_tap_table(const TcParams& p, const TileCoo
 // for the whole group (M = 128*CG, N = C_out), and each CTA drains its own 128 accumulator lanes.  When the
 // number of tiles is not a multiple of CG the last group's spare CTA runs a "ghost" copy of the last tile
 // and stores nothing.
-template <int MODE, typename T>
+template <int MODE, typename T, bool FD = false>
 __global__ void __launch_bounds__(tc_threads<MODE>(), 1)
 conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcParams p) {
+  static_assert(!FD || MODE == TC_PLAIN, "the FAM-decode epilogue belongs to the plain conv");
   using Cfg = TcCfg<MODE>;
   constexpr int CG = Cfg::CG, SA = Cfg::SA, SB = Cfg::SB;
   constexpr bool UNI = Cfg::UNIFIED;                   // B shares A's stage index and barriers
@@ -1176,6 +1183,22 @@ conv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
             emit_chunk(pk, 0.0f, 0.0f, 0.0f, 0.0f, c0 + TC_OUT_CH, ci + 1);
           }
         }
+      } else if (FD) {
+        // ---- FAM decode: this thread owns one pixel.  d_k = T(acc_k + bias_k) is bit for bit what the ordinary epilogue
+        // stores for channel k (and fam_decode_kernel reads back), and the decode is fam_decode_kernel's own code. ----
+        uint32_t v[32];
+        tmem_ld32(acc_addr, v);
+        release_acc();                                    // the deltas are in registers: the accumulator is free
+        if (valid) {
+          float d[5], a[5], o[5];
+#pragma unroll
+          for (int k = 0; k < 5; ++k) d[k] = round_through<T>(__uint_as_float(v[k]) + __ldg(bias + k));
+          fam_grid_anchor(x, y, L.stride, p.fd_scale, p.fd_angle, a);
+          delta2bbox_rotated<T>(a, d[0], d[1], d[2], d[3], d[4], p.fd_lim, o);
+          float* dst = L.refine + pos * 5;
+#pragma unroll
+          for (int k = 0; k < 5; ++k) dst[k] = o[k];
+        }
       } else if (IS_PLAIN && p.sc_tap >= 0) {
         // ---- dgrad: scatter the column gradient of tap sc_tap (this thread: one pixel, 32 channels at a time) ----
         const int H = L.H, W = L.W, t = p.sc_tap;
@@ -1467,10 +1490,10 @@ constexpr size_t tc_smem_bytes() {
          8 * TC_NBAR + 16;
 }
 
-template <int MODE, typename T>
+template <int MODE, typename T, bool FD = false>
 static int launch_tc(const TcMaps& tmap, const TcParams& p, cudaStream_t st) {
   constexpr int CG = TcCfg<MODE>::CG;
-  auto kern = conv_tc_kernel<MODE, T>;
+  auto kern = conv_tc_kernel<MODE, T, FD>;
   constexpr size_t smem = tc_smem_bytes<MODE>();
   static_assert(smem <= 227 * 1024, "shared memory budget");
   S2A_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1495,13 +1518,14 @@ static int launch_tc(const TcMaps& tmap, const TcParams& p, cudaStream_t st) {
 }
 
 struct TcScatter { float* gi; float* goff; const void* x; const void* off; int off_f32; int tap; };
+struct TcFamDecode { float* const* refined; float scale, angle, lim; };
 
 static int conv_tc_common(int mode, int nlevels, const void* const* xs, const float* const* anchors, const void* wp,
                           const float* bias, void* const* outs, void* const* pooleds, const int* Hs, const int* Ws,
                           const float* strides, int B, int C, int Co, int relu, int dtype, cudaStream_t st, int ks = 3,
                           int wsplit = -1, const void* wp2 = nullptr, const float* bias2 = nullptr,
                           const void* const* offsets = nullptr, int off_f32 = 0, int pos_round = 0,
-                          const TcScatter* sc = nullptr) {
+                          const TcScatter* sc = nullptr, const TcFamDecode* fd = nullptr) {
   if (wsplit < 0) wsplit = nlevels;              // one problem: every level uses the first weights
   S2A_CHECK_ARG(nlevels >= 1 && nlevels <= TC_MAX_LEVELS, "conv_tc: 1..%d levels per launch", TC_MAX_LEVELS);
   S2A_CHECK_ARG(B >= 0 && C > 0 && Co > 0, "conv_tc: bad tensor sizes");
@@ -1514,16 +1538,17 @@ static int conv_tc_common(int mode, int nlevels, const void* const* xs, const fl
   }
   const int Kp = ((C + TC_KB - 1) / TC_KB) * TC_KB * ks * ks;      // packed K' (C padded to 64-channel blocks)
   if (B == 0) return S2A_OK;
-  S2A_CHECK_ARG(xs && wp && outs && Hs && Ws, "conv_tc: null pointer");
+  S2A_CHECK_ARG(xs && wp && (fd ? fd->refined != nullptr : outs != nullptr) && Hs && Ws, "conv_tc: null pointer");
   TcParams p{};
   long long tiles = 0;
   for (int l = 0; l < nlevels; ++l) {
     S2A_CHECK_ARG(Hs[l] > 0 && Ws[l] > 0 && Hs[l] < 32768 && Ws[l] < 32768, "conv_tc: bad feature map size");
     S2A_CHECK_ARG((long long)Hs[l] * Ws[l] * C * 2 < (1ll << 32), "conv_tc: one image of a level must be < 4 GiB");
-    S2A_CHECK_ARG(xs[l] && outs[l] && (mode == TC_PLAIN || (anchors && anchors[l]) || (offsets && offsets[l])),
-                  "conv_tc: null level pointer");
+    S2A_CHECK_ARG(xs[l] && (fd ? fd->refined[l] != nullptr : outs[l] != nullptr) &&
+                  (mode == TC_PLAIN || (anchors && anchors[l]) || (offsets && offsets[l])), "conv_tc: null level pointer");
     TcLevel& L = p.lv[l];
-    L.x = xs[l]; L.anchors = anchors ? anchors[l] : nullptr; L.out = outs[l]; L.pooled = pooleds ? pooleds[l] : nullptr;
+    L.x = xs[l]; L.anchors = anchors ? anchors[l] : nullptr; L.out = outs ? outs[l] : nullptr;
+    L.pooled = pooleds ? pooleds[l] : nullptr; L.refine = fd ? fd->refined[l] : nullptr;
     L.offsets = offsets ? offsets[l] : nullptr;
     L.H = Hs[l]; L.W = Ws[l];
     const int pw = mode == TC_PLAIN ? TC_PPW : TC_PW, ph = mode == TC_PLAIN ? TC_PPH : TC_PH;
@@ -1531,7 +1556,7 @@ static int conv_tc_common(int mode, int nlevels, const void* const* xs, const fl
     if (l == wsplit) tiles += tiles & 1;         // the second problem starts at an even tile: pairs never mix weights
     L.tile_begin = (int)tiles;
     L.stride = strides ? strides[l] : 1.0f;
-    S2A_CHECK_ARG(mode == TC_PLAIN || L.stride > 0.0f, "alignconv_tc: stride must be positive");
+    S2A_CHECK_ARG((mode == TC_PLAIN && !fd) || L.stride > 0.0f, "conv_tc: stride must be positive");
     tiles += (long long)B * L.tiles_x * L.tiles_y;
   }
   S2A_CHECK_ARG(tiles < (1ll << 31), "conv_tc: too many tiles");
@@ -1555,7 +1580,7 @@ static int conv_tc_common(int mode, int nlevels, const void* const* xs, const fl
                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (xr != CUDA_SUCCESS) { set_error("conv_tc: cuTensorMapEncodeTiled (x, level %d) failed (%d)", l, (int)xr); return S2A_ERR_CUDA; }
   }
-  for (int l = 0; l < nlevels; ++l) {
+  for (int l = 0; l < nlevels && !fd; ++l) {         // (the FAM decode stores no feature map)
     const cuuint64_t yd[4] = {(cuuint64_t)Co, (cuuint64_t)Ws[l], (cuuint64_t)Hs[l], (cuuint64_t)B};
     const cuuint64_t ys_[3] = {(cuuint64_t)Co * 2, (cuuint64_t)Ws[l] * Co * 2, (cuuint64_t)Hs[l] * Ws[l] * Co * 2};
     const int pw = mode == TC_PLAIN ? TC_PPW : TC_PW;
@@ -1586,6 +1611,13 @@ static int conv_tc_common(int mode, int nlevels, const void* const* xs, const fl
     p.sc_gi = sc->gi; p.sc_goff = sc->goff; p.sc_x = sc->x; p.sc_off = sc->off; p.sc_off_f32 = sc->off_f32; p.sc_tap = sc->tap;
   }
   { const char* e = getenv("S2A_TC_DEBUG"); p.debug = e ? atoi(e) : 0; }
+  if (fd) {
+    S2A_CHECK_ARG(mode == TC_PLAIN && ks == 1 && Co == TC_OUT_CH && !relu && bias && !sc && !(pooleds && pooleds[0]),
+                  "conv_tc: bad FAM-decode arguments");
+    p.fd_scale = fd->scale; p.fd_angle = fd->angle; p.fd_lim = fd->lim;
+    return dtype == S2A_BF16 ? launch_tc<TC_PLAIN, __nv_bfloat16, true>(tmap, p, st)
+                             : launch_tc<TC_PLAIN, __half, true>(tmap, p, st);
+  }
   if (mode == TC_ALIGN) {
     return dtype == S2A_BF16 ? launch_tc<TC_ALIGN, __nv_bfloat16>(tmap, p, st) : launch_tc<TC_ALIGN, __half>(tmap, p, st);
   }
@@ -2450,4 +2482,21 @@ extern "C" int s2a_conv2d_forward_tc_multi2(int nlevels, int split, const void* 
   S2A_CHECK_ARG(packed_weight1 != nullptr, "conv2d_forward_tc_multi2: null pointer");
   return conv_tc_common(TC_PLAIN, nlevels, xs, nullptr, packed_weight0, bias0, outs, nullptr, Hs, Ws, nullptr, B, C, Co_pad,
                         relu, dtype, (cudaStream_t)stream, ks, split, packed_weight1, bias1);
+}
+
+// The FAM regression head (1 x 1, 5 output channels padded to 32, + bias; packed by s2a_conv2d_pack_weight) with the
+// anchor decode of s2a_fam_decode in its epilogue: refined[l] [B, H_l, W_l, 5] fp32, bit-identical to s2a_fam_decode of
+// the head's stored output; the deltas themselves are never written.
+extern "C" int s2a_conv2d_forward_tc_fam_decode(int nlevels, const void* const* xs, const void* packed_weight,
+                                                const float* bias, float* const* refined, const int* Hs, const int* Ws,
+                                                const float* strides, int B, int C, int Co_pad, float anchor_scale,
+                                                float anchor_angle, double wh_ratio_clip, int dtype, void* stream) {
+  using namespace s2a;
+  S2A_CHECK_ARG(Co_pad == TC_OUT_CH, "conv2d_forward_tc_fam_decode: the head must be padded to %d channels (got %d)",
+                TC_OUT_CH, Co_pad);
+  S2A_CHECK_ARG(bias && refined && strides, "conv2d_forward_tc_fam_decode: null pointer");
+  S2A_CHECK_ARG(wh_ratio_clip > 0.0, "conv2d_forward_tc_fam_decode: wh_ratio_clip must be positive");
+  const TcFamDecode fd{refined, anchor_scale, anchor_angle, clamp_limit(wh_ratio_clip, dtype)};
+  return conv_tc_common(TC_PLAIN, nlevels, xs, nullptr, packed_weight, bias, nullptr, nullptr, Hs, Ws, strides, B, C, Co_pad, 0,
+                        dtype, (cudaStream_t)stream, 1, -1, nullptr, nullptr, nullptr, 0, 0, nullptr, &fd);
 }

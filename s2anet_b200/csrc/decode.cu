@@ -8,11 +8,7 @@
 //   * get_bboxes_single_img up to (not including) the NMS: models/head.py:684-717 -- sigmoid,
 //     per-level top-k by best class score, gather, concatenation over levels, final
 //     delta2bbox_rotated; `s2a_select_decode` does all of it for the whole batch.
-// Arithmetic: models/boxes.py:82-162 (delta2bbox_rotated) and utils/general.py:925-930 (norm_angle),
-// operation by operation with individually rounded fp32 operations and the same dtype promotion as
-// PyTorch applies in the reference's half-precision validation (SURVEY Appendix A.7): anchors are
-// fp32, deltas are T; clamp / exp / pi*dangle are evaluated in T (rounded to T), everything that
-// touches an anchor value is fp32.
+// Arithmetic: box_decode.cuh (shared with the FAM-decode epilogue of conv_tc.cu).
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -20,6 +16,7 @@
 #include <type_traits>
 
 
+#include "box_decode.cuh"
 #include "common.cuh"
 
 namespace s2a {
@@ -59,38 +56,9 @@ __device__ __forceinline__ void load_channels(const T* q, long long cstride, lon
   }
 }
 
-// round a float through T (what storing a T tensor element does)
-template <typename T> __device__ __forceinline__ float round_through(float v);
-template <> __device__ __forceinline__ float round_through<float>(float v) { return v; }
-template <> __device__ __forceinline__ float round_through<__nv_bfloat16>(float v) {
-  return __bfloat162float(__float2bfloat16_rn(v));
-}
-template <> __device__ __forceinline__ float round_through<__half>(float v) { return __half2float(__float2half_rn(v)); }
-
 // torch.sigmoid on a T tensor: T(1 / (1 + exp(-float(x)))) (ATen UnarySpecialOpsKernel)
 template <typename T> __device__ __forceinline__ float sigmoid_t(float x) {
   return round_through<T>(__fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-x))));
-}
-
-// models/boxes.py:82-162 with is_encode_relative=True; a = (x, y, w, h, theta) fp32, d = deltas already
-// widened from T.  lim = max_ratio rounded to T (torch.clamp converts its bounds to the tensor dtype).
-template <typename T>
-__device__ __forceinline__ void delta2bbox_rotated(const float a[5], float dx, float dy, float dw, float dh, float da,
-                                                   float lim, float out[5]) {
-  dw = dw < -lim ? -lim : (dw > lim ? lim : dw);          // NaN stays NaN, like torch.clamp
-  dh = dh < -lim ? -lim : (dh > lim ? lim : dh);
-  const float cosa = cosf(a[4]), sina = sinf(a[4]);
-  const float dxw = __fmul_rn(dx, a[2]), dyh = __fmul_rn(dy, a[3]);
-  out[0] = __fadd_rn(__fsub_rn(__fmul_rn(dxw, cosa), __fmul_rn(dyh, sina)), a[0]);      // boxes.py:148
-  out[1] = __fadd_rn(__fadd_rn(__fmul_rn(dxw, sina), __fmul_rn(dyh, cosa)), a[1]);      // boxes.py:149
-  out[2] = __fmul_rn(a[2], round_through<T>(expf(dw)));                                 // boxes.py:155
-  out[3] = __fmul_rn(a[3], round_through<T>(expf(dh)));
-  const float kPi = 3.14159274101257324f, kQuarterPi = 0.785398185253143311f;           // float(np.pi), float(np.pi / 4)
-  const float ga = __fadd_rn(round_through<T>(__fmul_rn(da, kPi)), a[4]);               // boxes.py:159
-  // norm_angle (utils/general.py:925-930): (ga + pi/4) % pi - pi/4 with Python's sign convention
-  float m = fmodf(__fadd_rn(ga, kQuarterPi), kPi);
-  if (m != 0.0f && m < 0.0f) m = __fadd_rn(m, kPi);
-  out[4] = __fsub_rn(m, kQuarterPi);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -122,10 +90,8 @@ __global__ void __launch_bounds__(256) fam_decode_kernel(const __grid_constant__
     r /= L.W;
     const int y = (int)(r % L.H);
     const int b = (int)(r / L.H);
-    // models/anchors.py:94-95: centre = index * stride + 0.5 * (stride - 1); base size = scale * stride
-    const float half = __fmul_rn(0.5f, __fsub_rn(L.stride, 1.0f));
-    const float a[5] = {__fadd_rn(__fmul_rn((float)x, L.stride), half), __fadd_rn(__fmul_rn((float)y, L.stride), half),
-                        __fmul_rn(L.stride, p.scale), __fmul_rn(L.stride, p.scale), p.angle};
+    float a[5];
+    fam_grid_anchor(x, y, L.stride, p.scale, p.angle, a);
     const T* d = reinterpret_cast<const T*>(L.deltas) + b * L.s[0] + y * L.s[2] + x * L.s[3];
     float o[5];
     delta2bbox_rotated<T>(a, ld_as_float(d), ld_as_float(d + L.s[1]), ld_as_float(d + 2 * L.s[1]),
@@ -485,15 +451,6 @@ __global__ void __launch_bounds__(256) gather_decode_kernel(const __grid_constan
     float* gb = p.bboxes + row0 * 5;
     for (int e = tid; e < cnt * 5; e += 256) gb[e] = st_bb[e];
   }
-}
-
-template <typename T> static float limit_in(float max_ratio);
-template <> float limit_in<__nv_bfloat16>(float m) { return __bfloat162float(__float2bfloat16_rn(m)); }
-template <> float limit_in<__half>(float m) { return __half2float(__float2half_rn(m)); }
-
-static float clamp_limit(double wh_ratio_clip, int dtype) {
-  const float m = (float)fabs(log(wh_ratio_clip));           // boxes.py:115: np.abs(np.log(wh_ratio_clip))
-  return dtype == S2A_BF16 ? limit_in<__nv_bfloat16>(m) : dtype == S2A_F16 ? limit_in<__half>(m) : m;
 }
 
 template <typename T, int ITEMS>

@@ -31,6 +31,30 @@ def rboxes_decode(anchors, deltas, wh_ratio_clip=16 / 1000):
     return rboxes_decode_torch(anchors, deltas, wh_ratio_clip)
 
 
+# The 16-bit multi-level path: every conv is one persistent tcgen05 launch for all FPN levels (conv_tc).
+def _tc_conv(xs, m, relu=False):
+    from . import conv_tc
+    return conv_tc.conv2d_forward_tc_multi(xs, m.weight, m.bias, relu=relu)
+
+
+def _tc_tower(seq, xs):
+    for block in seq:                       # nn.Sequential(Conv2d, ReLU): one launch per layer for all levels
+        xs = _tc_conv(xs, block[0], relu=True)
+    return xs
+
+
+def _tc_pair(xs0, m0, xs1, m1, relu=False):      # two same-shaped convs in one launch (fills the CTA pairs better)
+    from . import conv_tc
+    return conv_tc.conv2d_forward_tc_pair(xs0, m0.weight, m0.bias, xs1, m1.weight, m1.bias, relu=relu)
+
+
+def _tc_towers(seq0, xs0, seq1, xs1):
+    """Two towers layer by layer; layers of the same shape class share a launch."""
+    for b0, b1 in zip(seq0, seq1):
+        xs0, xs1 = _tc_pair(xs0, b0[0], xs1, b1[0], relu=True)
+    return xs0, xs1
+
+
 class S2ANetHead(nn.Module):
     """Same sub-module / parameter names and constructor defaults as models/head.py:56-258."""
 
@@ -187,47 +211,51 @@ class S2ANetHead(nn.Module):
                                                   any(p.requires_grad for p in self.parameters()))
         if needs_grad or not (x0.is_cuda and x0.dtype in (torch.bfloat16, torch.float16) and self.with_orconv):
             return [self.forward_single(x, s) for x, s in zip(feats, self.featmap_strides)]
-        from . import conv_tc
-
-        def conv(xs, m, relu=False):
-            return conv_tc.conv2d_forward_tc_multi(xs, m.weight, m.bias, relu=relu)
-
-        def tower(seq, xs):
-            for block in seq:                       # nn.Sequential(Conv2d, ReLU): one launch per layer for all levels
-                xs = conv(xs, block[0], relu=True)
-            return xs
-
-        def pair(xs0, m0, xs1, m1, relu=False):      # two same-shaped convs in one launch (fills the CTA pairs better)
-            return conv_tc.conv2d_forward_tc_pair(xs0, m0.weight, m0.bias, xs1, m1.weight, m1.bias, relu=relu)
-
-        def towers(seq0, xs0, seq1, xs1):
-            """Two towers layer by layer; layers of the same shape class share a launch."""
-            for b0, b1 in zip(seq0, seq1):
-                xs0, xs1 = pair(xs0, b0[0], xs1, b1[0], relu=True)
-            return xs0, xs1
-
         feats = list(feats)
         if len(self.fam_reg_ls) == len(self.fam_cls_ls):
-            reg_feat, cls_feat = towers(self.fam_reg_ls, feats, self.fam_cls_ls, feats)
-            fam_reg, fam_cls = pair(reg_feat, self.fam_reg_head, cls_feat, self.fam_cls_head)
+            reg_feat, cls_feat = _tc_towers(self.fam_reg_ls, feats, self.fam_cls_ls, feats)
+            fam_reg, fam_cls = _tc_pair(reg_feat, self.fam_reg_head, cls_feat, self.fam_cls_head)
         else:
-            fam_reg = conv(tower(self.fam_reg_ls, feats), self.fam_reg_head)
-            fam_cls = conv(tower(self.fam_cls_ls, feats), self.fam_cls_head)
+            fam_reg = _tc_conv(_tc_tower(self.fam_reg_ls, feats), self.fam_reg_head)
+            fam_cls = _tc_conv(_tc_tower(self.fam_cls_ls, feats), self.fam_cls_head)
         refines = decode.fam_decode(fam_reg, self.featmap_strides, self.anchor_scale, self.anchor_angle, 1e-6)
+        odm_cls, odm_reg = self._odm_levels(feats, refines)
+        return [(fam_cls[l], fam_reg[l], odm_cls[l], odm_reg[l],
+                 self.grid_anchors(x.size(2), x.size(3), s, x.device), refines[l])
+                for l, (x, s) in enumerate(zip(feats, self.featmap_strides))]
+
+    def _odm_levels(self, feats, refines):
+        """AlignConv, ORConv and the ODM towers / heads of forward_levels' 16-bit path: (odm_cls, odm_reg) per level."""
+        from . import conv_tc
         aligned = conv_tc.alignconv_forward_tc_multi(feats, refines, self.align_conv.deform_conv.weight,
                                                      self.featmap_strides)
         or_feats, pooled = conv_tc.orconv_forward_tc_multi(aligned, self.or_conv.weight, self.or_conv.indices,
                                                            self.or_conv.bias, with_pool=True)
         if len(self.odm_cls_ls) == len(self.odm_reg_ls):
             # (the first layers differ in C -- 32 pooled vs 256 channels -- and fall back to two launches inside pair())
-            cls_feat, reg_feat = towers(self.odm_cls_ls, pooled, self.odm_reg_ls, or_feats)
-            odm_cls, odm_reg = pair(cls_feat, self.odm_cls_head, reg_feat, self.odm_reg_head)
-        else:
-            odm_cls = conv(tower(self.odm_cls_ls, pooled), self.odm_cls_head)
-            odm_reg = conv(tower(self.odm_reg_ls, or_feats), self.odm_reg_head)
-        return [(fam_cls[l], fam_reg[l], odm_cls[l], odm_reg[l],
-                 self.grid_anchors(x.size(2), x.size(3), s, x.device), refines[l])
-                for l, (x, s) in enumerate(zip(feats, self.featmap_strides))]
+            cls_feat, reg_feat = _tc_towers(self.odm_cls_ls, pooled, self.odm_reg_ls, or_feats)
+            return _tc_pair(cls_feat, self.odm_cls_head, reg_feat, self.odm_reg_head)
+        return (_tc_conv(_tc_tower(self.odm_cls_ls, pooled), self.odm_cls_head),
+                _tc_conv(_tc_tower(self.odm_reg_ls, or_feats), self.odm_reg_head))
+
+    def _forward_detect(self, feats):
+        """What detection reads, per level: (None, None, odm_cls, odm_reg, None, refine), or None where forward_levels
+        takes forward_single.  The FAM classification tower and head only feed the training loss, so they are not run:
+        two of the step's nine 256 -> 256 3x3 convs.  The regression tower layers run as single-problem launches instead
+        of paired with the classification ones, and the regression head decodes in its epilogue instead of storing deltas
+        for a fam_decode launch; every value is computed as forward_levels computes it, so the detections are
+        bit-identical to detect_from_outs(forward_levels(feats))."""
+        x0 = feats[0]
+        if torch.is_grad_enabled() or not (x0.is_cuda and x0.dtype in (torch.bfloat16, torch.float16) and self.with_orconv):
+            return None
+        from . import conv_tc
+        feats = list(feats)
+        # the regression head decodes its deltas into the refined anchors in its epilogue: bit for bit
+        # decode.fam_decode of its stored output, one launch and no delta tensor
+        refines = conv_tc.conv2d_forward_tc_fam_decode(_tc_tower(self.fam_reg_ls, feats), self.fam_reg_head,
+                                                       self.featmap_strides, self.anchor_scale, self.anchor_angle, 1e-6)
+        odm_cls, odm_reg = self._odm_levels(feats, refines)
+        return [(None, None, odm_cls[l], odm_reg[l], None, refines[l]) for l in range(len(feats))]
 
     @torch.no_grad()
     def select_and_decode(self, outs):
@@ -268,7 +296,7 @@ class S2ANetHead(nn.Module):
         """detect() with the detection exchange fused into the NMS finaliser: rows go straight into the packed
         [slots, max_per_img + 1, 8] buffers `dests` (tensors and / or NVLink peer pointers), image b at slot slot0 + b."""
         from .nms_rotated import multiclass_nms_rotated_packed
-        bboxes, scores = self.select_and_decode(self.forward_levels(feats))
+        bboxes, scores = self.select_and_decode(self._forward_detect(feats) or self.forward_levels(feats))
         multiclass_nms_rotated_packed(bboxes, scores, dests, slot0, self.score_thres_before_nms, self.iou_thres_nms,
                                       self.max_per_img, K=self.max_per_img)
 
@@ -276,7 +304,7 @@ class S2ANetHead(nn.Module):
     def detect(self, feats):
         """Whole hot path for a batch: head towers + AlignConv + ORConv + decode + multiclass NMS.
         Sync-free; returns (dets [B,max_per_img,6], labels [B,max_per_img], counts [B] int32)."""
-        return self.detect_from_outs(self.forward_levels(feats))
+        return self.detect_from_outs(self._forward_detect(feats) or self.forward_levels(feats))
 
     @torch.no_grad()
     def get_bboxes(self, feats):

@@ -199,8 +199,9 @@ static int by_score_desc(const void *a, const void *b)
  * labels == NULL -> class-agnostic (nms_rotated); otherwise pairs with different labels
  * never suppress (ml_nms_rotated/src/box_iou_rotated_utils.h:317-322, float equality).
  * ge != 0 selects the CPU build's  >=  predicate (nms_rotated_cpu.cpp:52).
- * The reference sort is not stable; ties are broken here by index (tests use distinct
- * scores).  Returns the number of kept boxes. */
+ * The reference sort is not stable; ties are broken here by index, lower first, which is
+ * the order the library's stable sorts give (tests/test_gpu_postprocess_exact.py checks it
+ * on tied 16-bit scores).  Returns the number of kept boxes. */
 S2A_API int64_t s2a_oracle_nms_rotated(const float *dets, const float *scores,
                                        const float *labels, int64_t n, float thr, int ge,
                                        int64_t *keep)

@@ -442,7 +442,8 @@ __device__ __forceinline__ void mc_select_sort_body(const float* __restrict__ sc
     if (i < n) {
       const float sv = sc[(int64_t)i * C + c];
       if (sv > thr) {
-        const unsigned u = __float_as_uint(sv);
+        // -0.0 and +0.0 are equal scores (ordered by box, like every other tie): one key for both
+        const unsigned u = sv == 0.0f ? 0u : __float_as_uint(sv);
         const unsigned ord = (u & 0x80000000u) ? ~u : (u | 0x80000000u);       // unsigned order == float order
         key[j] = ((unsigned long long)ord << 32) | (unsigned long long)(0xFFFFFFFFu - (unsigned)i);
         ++local;
@@ -473,10 +474,8 @@ __device__ __forceinline__ void mc_select_sort_body(const float* __restrict__ sc
   __syncthreads();
   for (int rank = threadIdx.x; rank < cnt; rank += kSelThreads) {
     const unsigned long long k = s_keys[rank];
-    const unsigned ord = (unsigned)(k >> 32);
-    const unsigned u = (ord & 0x80000000u) ? (ord & 0x7FFFFFFFu) : ~ord;
     const int box = (int)(0xFFFFFFFFu - (unsigned)(k & 0xFFFFFFFFull));
-    seg_score[rank] = __uint_as_float(u);
+    seg_score[rank] = sc[(int64_t)box * C + c];           // (the input's bits: the key has no sign of zero)
     seg_box[rank] = box;
     seg_rbox[rank] = prepped[box];
   }

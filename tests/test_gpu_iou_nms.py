@@ -160,9 +160,19 @@ def test_nms_keep_lists_golden(oracle, golden):
     np.testing.assert_array_equal(gpu_nms(b, s, 0.5, l), g["keep_mlnms_thr05_cuda_semantics"])
 
 
-@pytest.mark.parametrize("n_seed,rep,thr", [(1, 1, 0.5), (13, 5, 0.1), (50, 2, 0.7), (300, 7, 0.3), (1000, 3, 0.5)])
-def test_nms_vs_oracle(oracle, n_seed, rep, thr):
+_NMS_CASES = [(1, 1, 0.5), (13, 5, 0.1), (50, 2, 0.7), (300, 7, 0.3), (1000, 3, 0.5)]
+
+
+@pytest.mark.parametrize("n_seed,rep,thr,quantise", [pytest.param(*c, None, id="%d-%d-%g" % c) for c in _NMS_CASES] +
+                         [pytest.param(*c, q, id="%d-%d-%g-%s" % (c + (q,)))
+                          for c in [(300, 7, 0.3), (1000, 3, 0.5)] for q in ("bf16", "f16")])
+def test_nms_vs_oracle(oracle, n_seed, rep, thr, quantise):
+    """quantise: scores rounded through a 16-bit type, so that many are equal; equal scores keep their input order
+    (the generic path's stable sort), like the oracle's."""
     b, s, l = synth.clustered_boxes(n_seed=n_seed, rep=rep, seed=n_seed)
+    if quantise:
+        s = torch.from_numpy(s).to(torch.bfloat16 if quantise == "bf16" else torch.float16).float().numpy()
+        assert len(np.unique(s)) < 0.9 * len(s)
     np.testing.assert_array_equal(gpu_nms(b, s, thr), oracle.nms_rotated(b, s, thr))
     np.testing.assert_array_equal(gpu_nms(b, s, thr, l), oracle.nms_rotated(b, s, thr, labels=l))
 

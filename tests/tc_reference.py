@@ -1,13 +1,18 @@
-"""High-precision references for the 16-bit tensor-core convolutions (csrc/conv_tc.cu).
+"""High-precision references for the tensor-core and fp32 convolutions (csrc/conv_tc.cu, csrc/conv_f32.cu,
+csrc/deform_bwd.cu).
 
 * round_rne / ulp: correct round-to-nearest-even from float64 to bf16 / fp16.  torch's own float64 -> bf16 / fp16
   conversion goes through fp32 and so rounds twice (1 + 2**-8 + 2**-30 becomes 1.0 in bf16, not 1 + 2**-7).
 * check_budget: the condition under which a kernel that accumulates in fp32 -- in any order, including the tensor
   core's aligned partial sums -- must reproduce the exact result.
 * emulate_samples: the A operand the deformable (ALIGN) kernel builds, rounding for rounding.
+* tf32_split: the hi / lo TF32 split of the fp32 tensor-core kernel (cvt.rna.tf32.f32 twice).
+* geom_offsets / geom_positions / deform_grads_ref: offsets on a 1/4 grid and the float64 gradients for any kernel
+  size, stride, padding, dilation and (deformable) group count.
 
 Everything works on CPU and CUDA tensors alike.
 """
+import pytest
 import torch
 
 # precision (significand bits incl. the implicit one), minimum normal exponent, maximum exponent
@@ -160,3 +165,158 @@ def sampling_positions(offsets):
     h = offsets[:, 0::2] + (torch.arange(H, device=dev).view(1, 1, H, 1) - 1 + taps // 3)
     w = offsets[:, 1::2] + (torch.arange(W, device=dev).view(1, 1, 1, W) - 1 + taps % 3)
     return h, w
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# data and comparison shared by the exact tests
+# ------------------------------------------------------------------------------------------------------------------
+def ints(shape, r, g):
+    return torch.randint(-r, r + 1, tuple(shape), generator=g).double()
+
+
+def assert_exact(y, ref64, what):
+    """y (16-bit, or fp32) == ref64 rounded once to y's dtype; for fp32 y, ref64 must itself be an fp32 value.  On
+    failure: the count and the first mismatches with their (b, y, x, channel) for [B, C, H, W] tensors."""
+    ref64 = ref64.to(y.device)
+    if y.dtype in FORMATS:
+        want, got = round_rne(ref64, y.dtype), y
+    else:
+        assert bool((ref64.float().double() == ref64).all()), "%s: the float64 reference is not an fp32 value" % what
+        want, got = ref64, y.double()
+    bad = got != want
+    n = int(bad.sum())
+    if n == 0:
+        return
+    idx = bad.nonzero()[:5].tolist()
+    first = ", ".join("(b, y, x, c)=(%d, %d, %d, %d): got %r, want %r" % (i[0], i[2], i[3], i[1], float(got[tuple(i)]),
+                      float(want[tuple(i)])) if len(i) == 4 else "%s: got %r want %r" % (i, float(got[tuple(i)]),
+                      float(want[tuple(i)])) for i in idx)
+    raise AssertionError("%s: %d of %d outputs differ from the float64 reference; first %s" % (what, n, bad.numel(), first))
+
+
+def dyadic_anchors(B, H, W, stride, g):
+    """[B, H, W, 5] anchors whose tap positions the kernel computes exactly: angle 0 (cosf = 1, sinf = 0), centres on
+    a stride/4 grid, sizes 3 * stride * m / 4 (aw / 3.0f exact).  Centres move up to +-3 pixels, some by +-2.75 .. +-4
+    (corners leave the 14 x 22 halo), some anchors have zero size and some lie off the map."""
+    yy, xx = torch.meshgrid(torch.arange(H).double(), torch.arange(W).double(), indexing="ij")
+    a = torch.zeros(B, H, W, 5, dtype=torch.float64)
+    dx, dy = ints((B, H, W), 12, g) / 4, ints((B, H, W), 12, g) / 4
+    far = torch.tensor([2.75, 3.0, 3.25, 4.0, -2.75, -3.0, -3.25, -4.0], dtype=torch.float64)
+    pick = torch.rand(B, H, W, generator=g) < 0.25
+    dx = torch.where(pick, far[torch.randint(0, 8, (B, H, W), generator=g)], dx)
+    dy = torch.where(pick, far[torch.randint(0, 8, (B, H, W), generator=g)], dy)
+    a[..., 0], a[..., 1] = (xx + dx) * stride, (yy + dy) * stride
+    a[..., 2] = torch.randint(0, 13, (B, H, W), generator=g).double() * 3 * stride / 4
+    a[..., 3] = torch.randint(0, 13, (B, H, W), generator=g).double() * 3 * stride / 4
+    off_map = torch.rand(B, H, W, generator=g) < 0.03
+    a[..., 0] = torch.where(off_map, torch.full_like(a[..., 0], -6.0 * stride), a[..., 0])
+    return a
+
+
+def align_offsets(anchors, H, W, stride):
+    """[B, 18, H, W] AlignConv offsets of [B, H, W, 5] anchors, by the module's own get_offset (in anchors' dtype)."""
+    from s2anet_b200.alignconv import AlignConv
+    m = AlignConv(8, 8)
+    return torch.stack([m.get_offset(anchors[i].reshape(-1, 5), (H, W), stride) for i in range(anchors.size(0))])
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# the 3 x TF32 split (conv_tc.cu tf32_hi: cvt.rna.tf32.f32)
+# ------------------------------------------------------------------------------------------------------------------
+def tf32_round(v):
+    """fp32 -> the nearest TF32 value (10 explicit mantissa bits), ties away from zero, as an fp32 tensor with its low
+    13 bits zero: add half a TF32 step (0x1000) to the magnitude bits, clear the low 13 bits, keep the sign.  A carry
+    out of the mantissa moves the exponent up, as it should; subnormals round on the same bits."""
+    b = v.to(torch.float32).contiguous().view(torch.int32)
+    mag = b & 0x7FFFFFFF
+    r = ((mag + 0x1000) & ~0x1FFF) | (b & ~0x7FFFFFFF)
+    return r.view(torch.float32)
+
+
+def tf32_split(v):
+    """(hi, lo) of fp32 v: hi = tf32_round(v), lo = tf32_round(v - hi) (v - hi is exact in fp32).  hi + lo == v for
+    every v with at most 22 significant bits (unless lo is subnormal); for a TF32 tie (12 significant bits) lo is half a
+    TF32 step of v, with the sign opposite to v's."""
+    v = v.to(torch.float32)
+    hi = tf32_round(v)
+    return hi, tf32_round(v - hi)
+
+
+def odd_fractions(shape, g):
+    """fp64 values +-(1 + m 2**-11), m odd in [1, 2047]: 12 significant bits, so every one is a TF32 tie whose lo part is
+    +-2**-11."""
+    m = 2 * torch.randint(0, 1024, tuple(shape), generator=g) + 1
+    s = torch.where(torch.rand(tuple(shape), generator=g) < 0.5, -1.0, 1.0).double()
+    return s * (1.0 + m.double() * 2.0 ** -11)
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# deformable geometry: any kernel size, stride, padding, dilation, deformable groups
+# ------------------------------------------------------------------------------------------------------------------
+def out_size(n, k, stride, pad, dil):
+    return (n + 2 * pad - (dil * (k - 1) + 1)) // stride + 1
+
+
+def _tap_bases(Ho, Wo, k, stride, pad, dil, dev=None):
+    """Regular-grid positions [k*k, Ho, 1] (rows) and [k*k, 1, Wo] (columns) of each tap: ho*stride - pad + i*dil."""
+    taps = torch.arange(k * k, device=dev).view(k * k, 1, 1)
+    bh = torch.arange(Ho, device=dev).view(1, Ho, 1) * stride - pad + (taps // k) * dil
+    bw = torch.arange(Wo, device=dev).view(1, 1, Wo) * stride - pad + (taps % k) * dil
+    return bh, bw
+
+
+# (h, w) that every geom_offsets draw contains: exactly -1, just inside -1, exactly (H - 1, W - 1), inside (W - 1, W),
+# the far corner just inside the map, and a position inside -1 on both axes
+EDGE_POSITIONS = lambda H, W: ((-1.0, 0.5), (-0.75, 0.25), (H - 1.0, W - 1.0), (0.5, W - 0.75), (H - 0.25, W - 0.25),
+                               (-0.25, -0.75))
+
+
+def geom_offsets(B, H, W, k, stride, pad, dil, dgroups, g, spread=2.0):
+    """[B, dgroups*2*k*k, Ho, Wo] float64 offsets on a 1/4 grid for a k x k deformable conv (CPU, from generator g), in
+    the reference's layout (deformable group, tap, (dy, dx)).  As quarter_offsets: half of the positions are the regular
+    grid moved by up to `spread` pixels, half anywhere in [-3, H + 0.25] x [-3, W + 0.25]; and in every deformable
+    group the first pixels carry EDGE_POSITIONS (entry s at tap s % k*k, pixel s // k*k in raster order)."""
+    Ho, Wo = out_size(H, k, stride, pad, dil), out_size(W, k, stride, pad, dil)
+    kk = k * k
+    bh, bw = (t.double() for t in _tap_bases(Ho, Wo, k, stride, pad, dil))
+    off = torch.randint(int(-4 * spread), int(4 * spread) + 1, (B, dgroups, kk, 2, Ho, Wo), generator=g).double() / 4
+    hh = torch.randint(-8, 4 * H + 5, (B, dgroups, kk, Ho, Wo), generator=g).double() / 4 - 1
+    ww = torch.randint(-8, 4 * W + 5, (B, dgroups, kk, Ho, Wo), generator=g).double() / 4 - 1
+    pick = torch.rand(B, dgroups, kk, Ho, Wo, generator=g) < 0.5
+    off[:, :, :, 0] = torch.where(pick, hh - bh, off[:, :, :, 0])
+    off[:, :, :, 1] = torch.where(pick, ww - bw, off[:, :, :, 1])
+    edges = EDGE_POSITIONS(H, W)
+    assert Ho * Wo * kk >= len(edges), "geom_offsets: too few (pixel, tap) pairs for the edge positions"
+    for s, (ph, pw) in enumerate(edges):
+        t, (ho, wo) = s % kk, divmod(s // kk, Wo)
+        off[0, :, t, 0, ho, wo] = ph - float(bh[t, ho, 0])
+        off[0, :, t, 1, ho, wo] = pw - float(bw[t, 0, wo])
+    return off.reshape(B, dgroups * 2 * kk, Ho, Wo)
+
+
+def geom_positions(off, k, stride, pad, dil):
+    """(h, w) [B, dgroups, k*k, Ho, Wo] of [B, dgroups*2*k*k, Ho, Wo] offsets, in the offsets' dtype and device."""
+    B, ch, Ho, Wo = off.shape
+    o = off.view(B, ch // (2 * k * k), k * k, 2, Ho, Wo)
+    bh, bw = _tap_bases(Ho, Wo, k, stride, pad, dil, off.device)
+    return o[:, :, :, 0] + bh, o[:, :, :, 1] + bw
+
+
+def deform_grads_ref(x, off, w, go, stride=1, pad=1, dil=1):
+    """torchvision's float64 autograd: (grad_input, grad_offset, grad_weight), with the offset gradient of a sampling
+    position outside -1 < h < H, -1 < w < W set to 0.  That is the reference DCN's rule (its coordinate-weight kernel
+    moves such positions to -2, where no corner is inside the map) and the one this repository's fp32 col2im and the
+    tcgen05 dgrad follow.  torchvision differs only at h == -1 or w == -1 exactly: the sample is 0 there and its
+    right-hand derivative is not, and torchvision returns that derivative.  Groups and deformable groups follow from
+    the shapes of w and off, as in torchvision."""
+    tv = pytest.importorskip("torchvision")
+    x64 = x.detach().double().clone().requires_grad_(True)          # (a copy even when x already is float64)
+    off64 = off.detach().to(x.device).double().clone().requires_grad_(True)
+    w64 = w.detach().to(x.device).double().clone().requires_grad_(True)
+    tv.ops.deform_conv2d(x64, off64, w64, stride=stride, padding=pad, dilation=dil).backward(go.to(x.device).double())
+    H, W = x.shape[2:]
+    h, ww = geom_positions(off64.detach(), w.size(-1), stride, pad, dil)
+    outside = ~((h > -1) & (ww > -1) & (h < H) & (ww < W))                     # [B, dg, kk, Ho, Wo]
+    outside = outside.unsqueeze(3).expand(-1, -1, -1, 2, -1, -1).reshape(off64.shape)
+    goff = torch.where(outside, torch.zeros_like(off64.grad), off64.grad)
+    return x64.grad, goff, w64.grad

@@ -17,8 +17,8 @@ import torch
 import torch.nn.functional as F
 
 from s2anet_b200 import synth
-from tc_reference import (FORMATS, check_budget, contract_samples, emulate_samples, quarter_offsets, round_rne,
-                          sampling_positions, ulp)
+from tc_reference import (FORMATS, align_offsets, assert_exact, check_budget, contract_samples, deform_grads_ref, dyadic_anchors,
+                          emulate_samples, ints, quarter_offsets, round_rne, sampling_positions, ulp)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -39,29 +39,8 @@ def tv():
     return pytest.importorskip("torchvision")
 
 
-def ints(shape, r, g):
-    return torch.randint(-r, r + 1, tuple(shape), generator=g).double()
-
-
 def cl(t, dtype):
     return t.to(DEV).to(dtype).contiguous(memory_format=torch.channels_last)
-
-
-def assert_exact(y, ref64, what):
-    """y (16-bit, or fp32 for the gradients) == ref64 rounded once to y's dtype.  On failure: the count and the first
-    mismatches with their (b, y, x, channel) for [B, C, H, W] tensors."""
-    ref64 = ref64.to(y.device)
-    want = round_rne(ref64, y.dtype) if y.dtype in FORMATS else ref64
-    got = y if y.dtype in FORMATS else y.double()
-    bad = got != want
-    n = int(bad.sum())
-    if n == 0:
-        return
-    idx = bad.nonzero()[:5].tolist()
-    first = ", ".join("(b, y, x, c)=(%d, %d, %d, %d): got %r, want %r" % (i[0], i[2], i[3], i[1], float(got[tuple(i)]),
-                      float(want[tuple(i)])) if len(i) == 4 else "%s: got %r want %r" % (i, float(got[tuple(i)]),
-                      float(want[tuple(i)])) for i in idx)
-    raise AssertionError("%s: %d of %d outputs differ from the float64 reference; first %s" % (what, n, bad.numel(), first))
 
 
 def assert_exact_blend(x, dtype, what):
@@ -188,31 +167,6 @@ def deform_ref(x, off, w, relu):
     return (ref.relu() if relu else ref), S
 
 
-def dyadic_anchors(B, H, W, stride, g):
-    """[B, H, W, 5] anchors whose tap positions the kernel computes exactly: angle 0 (cosf = 1, sinf = 0), centres on
-    a stride/4 grid, sizes 3 * stride * m / 4 (aw / 3.0f exact).  Centres move up to +-3 pixels, some by +-2.75 .. +-4
-    (corners leave the 14 x 22 halo), some anchors have zero size and some lie off the map."""
-    yy, xx = torch.meshgrid(torch.arange(H).double(), torch.arange(W).double(), indexing="ij")
-    a = torch.zeros(B, H, W, 5, dtype=torch.float64)
-    dx, dy = ints((B, H, W), 12, g) / 4, ints((B, H, W), 12, g) / 4
-    far = torch.tensor([2.75, 3.0, 3.25, 4.0, -2.75, -3.0, -3.25, -4.0], dtype=torch.float64)
-    pick = torch.rand(B, H, W, generator=g) < 0.25
-    dx = torch.where(pick, far[torch.randint(0, 8, (B, H, W), generator=g)], dx)
-    dy = torch.where(pick, far[torch.randint(0, 8, (B, H, W), generator=g)], dy)
-    a[..., 0], a[..., 1] = (xx + dx) * stride, (yy + dy) * stride
-    a[..., 2] = torch.randint(0, 13, (B, H, W), generator=g).double() * 3 * stride / 4
-    a[..., 3] = torch.randint(0, 13, (B, H, W), generator=g).double() * 3 * stride / 4
-    off_map = torch.rand(B, H, W, generator=g) < 0.03
-    a[..., 0] = torch.where(off_map, torch.full_like(a[..., 0], -6.0 * stride), a[..., 0])
-    return a
-
-
-def align_offsets(anchors, H, W, stride):
-    from s2anet_b200.alignconv import AlignConv
-    m = AlignConv(8, 8)
-    return torch.stack([m.get_offset(anchors[i].reshape(-1, 5), (H, W), stride) for i in range(anchors.size(0))])
-
-
 def check_align(entry, dtype, x, anc, w, stride, y, what):
     off = align_offsets(anc.double(), x.size(2), x.size(3), stride)
     assert_quarter_grid(off, what)
@@ -299,23 +253,6 @@ def test_deform_conv_forward_cuda_half_exact(dtype):
     ref, S = deform_ref(x, off, wt, False)
     check_budget(S, 1 / 16, dtype, ref, "deform_conv_forward_cuda %s" % dtype)
     assert_exact(out, ref, "deform_conv_forward_cuda %s" % dtype)
-
-
-def deform_grads_ref(x, off, w, go):
-    """torchvision's float64 autograd: (grad_input, grad_offset, grad_weight), with the offset gradient of a sampling
-    position outside -1 < h < H, -1 < w < W set to 0.  That is the reference DCN's rule (its coordinate-weight kernel
-    moves such positions to -2, where no corner is inside the map) and the one this repository's fp32 col2im and the
-    tcgen05 dgrad follow.  torchvision differs only at h == -1 or w == -1 exactly: the sample is 0 there and its
-    right-hand derivative is not, and torchvision returns that derivative."""
-    x64 = x.double().requires_grad_(True)
-    off64 = off.to(x.device).double().requires_grad_(True)
-    w64 = w.to(x.device).double().requires_grad_(True)
-    tv().ops.deform_conv2d(x64, off64, w64, padding=1).backward(go.double())
-    H, W = x.shape[2:]
-    h, ww = sampling_positions(off64.detach())
-    outside = ~((h > -1) & (ww > -1) & (h < H) & (ww < W))
-    goff = torch.where(outside.repeat_interleave(2, dim=1), torch.zeros_like(off64.grad), off64.grad)
-    return x64.grad, goff, w64.grad
 
 
 @pytest.mark.parametrize("dtype", DTYPES)

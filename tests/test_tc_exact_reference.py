@@ -1,10 +1,11 @@
 """CPU checks of the references in tc_reference.py, which the exact and rounding-model tests of the 16-bit tensor-core
-convolutions (test_gpu_tc_exact.py) rest on."""
+convolutions (test_gpu_tc_exact.py) and the fp32 convolutions (test_gpu_fp32_exact.py) rest on."""
 import numpy as np
 import pytest
 import torch
 
-from tc_reference import FORMATS, check_budget, emulate_samples, quarter_offsets, round_rne, round_rne64, ulp
+from tc_reference import (EDGE_POSITIONS, FORMATS, check_budget, emulate_samples, geom_offsets, geom_positions, odd_fractions,
+                          out_size, quarter_offsets, round_rne, round_rne64, sampling_positions, tf32_round, tf32_split, ulp)
 
 BF16, F16 = torch.bfloat16, torch.float16
 
@@ -125,3 +126,89 @@ def test_emulate_samples_models_rounding():
     xr = torch.randn(1, 8, 6, 9, generator=g).to(BF16)
     _, inexact = emulate_samples(xr, torch.randn(1, 18, 6, 9, generator=g) * 1.5, BF16, False, return_inexact=True)
     assert inexact > 0
+
+
+def _f32bits(t):
+    return t.to(torch.float32).contiguous().view(torch.int32)
+
+
+def test_tf32_split_ties_round_away_from_zero():
+    """cvt.rna: a tie goes away from zero.  Round-to-nearest-even would give 1, -1 and 1 + 2**-9 here."""
+    v = torch.tensor([1 + 2 ** -11, -(1 + 2 ** -11), 1 + 3 * 2 ** -11, 2 - 2 ** -11, 1 + 2 ** -11 - 2 ** -20,
+                      1 + 2 ** -11 + 2 ** -20], dtype=torch.float64)
+    want = [1 + 2 ** -10, -(1 + 2 ** -10), 1 + 2 ** -9, 2.0, 1.0, 1 + 2 ** -10]
+    hi, lo = tf32_split(v.float())
+    assert hi.double().tolist() == want
+    assert torch.equal(hi.double() + lo.double(), v)
+    assert lo.double().tolist()[:4] == [-2 ** -11, 2 ** -11, -2 ** -11, -2 ** -11]
+
+
+def test_tf32_split_is_exact_below_23_bits():
+    """hi + lo == v for every v with at most 22 significant bits whose lo part is not subnormal (a subnormal lo is
+    rounded on its own, coarser bits); hi and lo are TF32 values (low 13 bits zero)."""
+    g = torch.Generator().manual_seed(7)
+    m = torch.randint(2 ** 21, 2 ** 22, (20000,), generator=g).double()
+    e = torch.randint(-100, 100, (20000,), generator=g).double()
+    s = torch.where(torch.rand(20000, generator=g) < 0.5, -1.0, 1.0).double()
+    v = (s * m * torch.pow(2.0, e - 21)).float()
+    hi, lo = tf32_split(v)
+    assert torch.equal(hi.double() + lo.double(), v.double())
+    assert bool(((_f32bits(hi) & 0x1FFF) == 0).all()) and bool(((_f32bits(lo) & 0x1FFF) == 0).all())
+    assert bool((lo.double().abs() <= torch.pow(2.0, torch.floor(torch.log2(hi.double().abs())) - 11)).all())
+    # 24-bit values: the residual v - hi - lo is what the kernel drops, at most 2**-22 |v|
+    w = torch.randn(20000, generator=g)
+    hw, lw = tf32_split(w)
+    res = (w.double() - hw.double() - lw.double()).abs()
+    assert bool((res <= 2.0 ** -22 * w.double().abs()).all()) and bool((res > 0).any())
+
+
+def test_tf32_split_zeros_and_subnormals():
+    z = torch.tensor([0.0, -0.0])
+    hi, lo = tf32_split(z)
+    assert _f32bits(hi).tolist() == _f32bits(z).tolist()                 # the sign of zero survives in hi
+    assert _f32bits(lo).tolist() == [0, 0]                               # -0 - -0 = +0
+    # subnormals round on the same bits: 0x1FFF -> 0x2000 (up), 0x0FFF -> 0 (down), 0x1000 -> 0x2000 (tie, away)
+    bits = torch.tensor([0x1FFF, 0x0FFF, 0x1000, 0x3000, 0x7FFFFF, 0x00400000 | 0x1000], dtype=torch.int32)
+    sub = bits.view(torch.float32)
+    hi, lo = tf32_split(sub)
+    assert _f32bits(hi).tolist() == [0x2000, 0, 0x2000, 0x4000, 0x800000, 0x00402000]
+    # the residuals are subnormal too and round likewise (-1 bit becomes -0): hi + lo need not equal v down here
+    neg = lambda b: b - 2 ** 32 if b >= 2 ** 31 else b
+    assert _f32bits(lo).tolist() == [neg(0x80000000), 0, neg(0x80002000), neg(0x80002000), neg(0x80000000), neg(0x80002000)]
+    assert torch.equal(_f32bits(tf32_round(-sub)), _f32bits(-hi))
+    # a carry out of the mantissa moves the exponent: the largest value below 2 rounds to 2
+    assert float(tf32_round(torch.tensor([2 - 2 ** -23]))) == 2.0
+
+
+def test_odd_fractions_are_tf32_ties():
+    g = torch.Generator().manual_seed(8)
+    v = odd_fractions((5000,), g)
+    assert bool(((v.abs() > 1) & (v.abs() < 2)).all())
+    hi, lo = tf32_split(v.float())
+    assert torch.equal(v.float().double(), v)
+    assert torch.equal(lo.double().abs(), torch.full_like(v, 2.0 ** -11))
+    assert torch.equal(torch.sign(lo.double()), -torch.sign(v))          # hi is the neighbour away from zero
+
+
+@pytest.mark.parametrize("k,stride,pad,dil,dgroups", [(3, 1, 1, 1, 1), (3, 2, 2, 2, 2), (1, 2, 0, 1, 1), (2, 1, 0, 1, 1),
+                                                      (3, 1, 0, 1, 4), (5, 1, 2, 1, 1), (7, 2, 3, 1, 1)])
+def test_geom_offsets_hit_the_edges(k, stride, pad, dil, dgroups):
+    """Every draw puts positions exactly on -1, just inside -1, exactly on H - 1 and W - 1, inside (W - 1, W), and off
+    the map, in every deformable group; everything lies on the 1/4 grid."""
+    g = torch.Generator().manual_seed(k + stride + dgroups)
+    B, H, W = 2, 9, 11
+    off = geom_offsets(B, H, W, k, stride, pad, dil, dgroups, g)
+    Ho, Wo = out_size(H, k, stride, pad, dil), out_size(W, k, stride, pad, dil)
+    assert tuple(off.shape) == (B, dgroups * 2 * k * k, Ho, Wo)
+    assert torch.equal(off * 4, (off * 4).round())
+    h, w = geom_positions(off, k, stride, pad, dil)
+    for d in range(dgroups):
+        hd, wd = h[:, d], w[:, d]
+        assert (hd == -1).any() and (hd == -0.75).any() and (hd == H - 1).any() and (wd == W - 1).any()
+        assert ((wd > W - 1) & (wd < W)).any() and ((hd <= -1) | (hd >= H) | (wd <= -1) | (wd >= W)).any()
+        for s, (ph, pw) in enumerate(EDGE_POSITIONS(H, W)):
+            t, (ho, wo) = s % (k * k), divmod(s // (k * k), Wo)
+            assert (float(hd[0, t, ho, wo]), float(wd[0, t, ho, wo])) == (ph, pw)
+    if (k, stride, pad, dil) == (3, 1, 1, 1) and dgroups == 1:            # the 3x3 / pad 1 positions agree
+        hs, ws = sampling_positions(off)
+        assert torch.equal(hs, h[:, 0]) and torch.equal(ws, w[:, 0])

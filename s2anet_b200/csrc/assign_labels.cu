@@ -12,6 +12,8 @@
 //           (the reference loops GTs in ascending order, :130-144), then the positive / negative rules.
 // Pairs proven disjoint have IoU exactly 0 and take part in neither maximum that matters (a row maximum of 0
 // only tells "negative" from "ignored", which the count of valid pairs decides).
+#include <climits>
+
 #include "common.cuh"
 #include "rbox_iou.cuh"
 
@@ -23,9 +25,9 @@ struct AssignParams {
   const float* anchors;      // [B, M, 5]
   const float* gts;          // [B, Nmax, 5]
   const int32_t* gt_counts;  // [B] or null (= Nmax everywhere)
-  unsigned long long* col_best;   // [B, Nmax] packed (IoU bits << 32 | ~anchor index), zeroed before pass 1
+  unsigned long long* col_best;   // [B, Nmax] packed (IoU bits << 32 | ~anchor index), zeroed before pass 1; ~0 = a NaN IoU
   unsigned long long* row_best;   // [B, M] packed (IoU bits + 1 << 32 | ~gt index); 0 = no positive IoU
-  int32_t* row_bad;          // [B, M] number of (valid-anchor) pairs whose IoU fell outside [0, 1]
+  int32_t* row_bad;          // [B, M] number of (valid-anchor) pairs whose IoU fell outside [0, 1]; sign bit: a NaN IoU
   int64_t* assign;           // [B, M]
   long long M, Nmax;
   float img_w, img_h, pos_thr, neg_thr, min_pos_thr;
@@ -134,6 +136,13 @@ __global__ void __launch_bounds__(kAsgThreads) assign_labels_kernel(const Assign
       bool ok;
       float v = rbox_iou_clip_try(s_row[r], s_col[c], s_pts + tid, kAsgThreads, ok);
       if (!ok) v = asg_clip_general(s_row[r], s_col[c]);
+      if (v != v) {
+        // A NaN IoU passes the range filter (models/utils.py:89-96) and propagates through torch.max: the row maximum
+        // is NaN (neither negative nor positive), and so is the GT's maximum (no anchor is forced onto it).  Marked by
+        // the sign bit of the row's count, and by a column key above every IoU key.
+        if (PASS == 1) { atomicOr(&s_rbad[r], INT_MIN); atomicMax(&s_cbest[c], ~0ull); }
+        continue;
+      }
       if (!(v >= 0.0f && v <= 1.0f)) {                  // models/utils.py:89-96: out-of-range IoUs become -0.5
         if (PASS == 1) atomicAdd(&s_rbad[r], 1);
         continue;
@@ -167,15 +176,18 @@ __global__ void __launch_bounds__(kAsgThreads) assign_labels_kernel(const Assign
         if (ngt == 0) {
           res = -1;                                      // :79-86: no GT at all -> every valid anchor is negative
         } else {
-          const unsigned long long rb = p.row_best[a];
-          const int nvalid = ngt - p.row_bad[a];         // pairs with an IoU in [0, 1]
-          // row maximum: the best positive IoU, else 0 if any pair is valid, else -0.5
-          const float mx = rb ? __uint_as_float((unsigned)(rb >> 32) - 1u) : (nvalid > 0 ? 0.0f : -0.5f);
-          if (mx >= 0.0f && mx < p.neg_thr) res = -1;    // :116
-          if (mx >= p.pos_thr) {                         // :122-123 (argmax = first index of the maximum)
-            if (rb) res = (long long)(0xFFFFFFFFu - (unsigned)(rb & 0xFFFFFFFFull));
-            else {                                       // maximum 0 reached the positive threshold (pos_thr <= 0): first valid pair
-              res = 0;
+          const int bad = p.row_bad[a];
+          if (bad >= 0) {                                // (< 0: a NaN IoU in the row, its maximum is NaN: ignored)
+            const unsigned long long rb = p.row_best[a];
+            const int nvalid = ngt - bad;                // pairs with an IoU in [0, 1]
+            // row maximum: the best positive IoU, else 0 if any pair is valid, else -0.5
+            const float mx = rb ? __uint_as_float((unsigned)(rb >> 32) - 1u) : (nvalid > 0 ? 0.0f : -0.5f);
+            if (mx >= 0.0f && mx < p.neg_thr) res = -1;  // :116
+            if (mx >= p.pos_thr) {                       // :122-123 (argmax = first index of the maximum)
+              if (rb) res = (long long)(0xFFFFFFFFu - (unsigned)(rb & 0xFFFFFFFFull));
+              else {                                     // maximum 0 reached the positive threshold (pos_thr <= 0): first valid pair
+                res = 0;
+              }
             }
           }
           if (s_match[tid] >= 0) res = s_match[tid];     // :130-144

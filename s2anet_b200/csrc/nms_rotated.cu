@@ -152,20 +152,8 @@ __device__ __forceinline__ void mask_tile_warp(WarpTileSmem& s, const RBox* __re
         if (rbox_classify(rb, cb) == RB_ZERO) {
           if (0.0f > thr) atomicOr(reinterpret_cast<unsigned*>(&s.word[p >> 6]) + ((p >> 5) & 1), 1u << (p & 31));
         } else {
-          // The sweep only needs "IoU > thr".  intersection <= min(area) and union >= max(area), so a pair whose area
-          // ratio is below thr (with 0.1 % slack for the reference's fp32 polygon area) cannot suppress: no clip.
-          const float ar = rb.w * rb.h, ac = cb.w * cb.h;
-          bool small = false;
-          if (thr > 0.0f && rb.w > 0.0f && rb.h > 0.0f && cb.w > 0.0f && cb.h > 0.0f) {
-            small = fminf(ar, ac) < 0.999f * thr * fmaxf(ar, ac);
-            if (!small) {
-              // tighter: the overlap of each box with the other's axis-aligned extent in its own frame (0.1 % slack
-              // again); IoU <= ub / (a1 + a2 - ub) is increasing in ub
-              const float ub = 1.001f * rbox_inter_upper_bound(rb, cb);
-              small = ub < 0.999f * thr * (ar + ac - ub);
-            }
-          }
-          clip = !small;
+          // the sweep only needs "IoU > thr": no clip for a pair whose IoU provably cannot exceed it
+          clip = !rbox_nms_cannot_exceed(rb, cb, thr);
         }
       }
       const unsigned bal = __ballot_sync(0xffffffffu, clip);

@@ -134,6 +134,19 @@ RB_HD bool rbox_fast_zero(const RFast& A, const RAng& aA, const RFast& B, const 
   return (dx * dx + dy * dy > 1.21f * rs * rs) && (fabsf(s2d) > 0.02f) && (fminf(A.mn, B.mn) > RB_SLIVER * ext);
 }
 
+// Near-parallel (C >= S) or near-perpendicular pairs: every pair of parallel edge lines is more than g apart,
+// measured through the centres in A's frame (B's half extents along A's axes; duA, dvA: the centre offset there).
+RB_HD bool rbox_parallel_edges_apart(const RBox& A, const RBox& B, float duA, float dvA, float S, float C, float g) {
+  const float wB = fabsf(B.w), hB = fabsf(B.h);
+  const float bu = 0.5f * (C >= S ? wB : hB), bv = 0.5f * (C >= S ? hB : wB);
+  const float au = 0.5f * fabsf(A.w), av = 0.5f * fabsf(A.h);
+  const float gv = fminf(fminf(fabsf(dvA + bv - av), fabsf(dvA + bv + av)),
+                         fminf(fabsf(dvA - bv - av), fabsf(dvA - bv + av)));
+  const float gu = fminf(fminf(fabsf(duA + bu - au), fabsf(duA + bu + au)),
+                         fminf(fabsf(duA - bu - au), fabsf(duA - bu + au)));
+  return gv > g && gu > g;
+}
+
 RB_HD int rbox_classify(const RBox& A, const RBox& B) {
   float a1 = RB_MUL(A.w, A.h), a2 = RB_MUL(B.w, B.h);
   if (a1 <= RB_LO_1E14 || a2 <= RB_LO_1E14) return RB_ZERO;     // (double)area < 1e-14
@@ -163,14 +176,7 @@ RB_HD int rbox_classify(const RBox& A, const RBox& B) {
   if (sep && mnp > RB_SLIVER * ext && gap * mnp > RB_GAPRULE * ext * ext) {
     // |sd*cd| = |sin(2 dT)|/32
     if (fabsf(sd * cd) > 0.000625f) return RB_ZERO;
-    // near-parallel (C >= S) or near-perpendicular: B's half extents along A's axes
-    const float bu = 0.5f * (C >= S ? wB : hB), bv = 0.5f * (C >= S ? hB : wB);
-    const float au = 0.5f * wA, av = 0.5f * hA, g = 0.1f * ext;
-    const float gv = fminf(fminf(fabsf(dvA + bv - av), fabsf(dvA + bv + av)),
-                           fminf(fabsf(dvA - bv - av), fabsf(dvA - bv + av)));
-    const float gu = fminf(fminf(fabsf(duA + bu - au), fabsf(duA + bu + au)),
-                           fminf(fabsf(duA - bu - au), fabsf(duA - bu + au)));
-    if (gv > g && gu > g) return RB_ZERO;
+    if (rbox_parallel_edges_apart(A, B, duA, dvA, S, C, 0.1f * ext)) return RB_ZERO;
   }
   return RB_CLIP;
 }
@@ -192,6 +198,44 @@ RB_HD float rbox_inter_upper_bound(const RBox& A, const RBox& B) {
   const float ouB = fmaxf(0.0f, fminf(0.5f * B.w, euB - duB) - fmaxf(-0.5f * B.w, -duB - euB));
   const float ovB = fmaxf(0.0f, fminf(0.5f * B.h, evB - dvB) - fmaxf(-0.5f * B.h, -dvB - evB));
   return fminf(fminf(ouA * ovA, ouB * ovB), fminf(A.w * A.h, B.w * B.h));
+}
+
+// NMS clip skip: true only if the reference's IoU of the pair cannot exceed thr, so the suppression bit is 0 without
+// clipping.  Geometrically, inter <= min(area) and union >= max(area), and IoU <= ub / (a1 + a2 - ub) with ub the
+// bound above; both tests keep 0.1 % slack on each side for the reference's fp32 arithmetic.  That slack only holds
+// where the reference computes the polygon well, so the shortcut takes conditions of the kind rbox_classify takes:
+//   * Sliver guard.  Vertex coordinates are off by eps_v <= 2^-22 * ext.  A polygon vertex that moves by d along its
+//     own edge changes the area by <= d * L * sin(phi) / 2, and a crossing at angle phi is off by ~eps_v / sin(phi)
+//     along the edge, so every vertex and every fan triangle adds ~eps_v * L.  The intersection error is then about
+//     4 eps_v times the smaller box's perimeter 2 (a + b) <= 4 a (sides a >= b).  An intersection that can reach thr
+//     is >= thr * max area >= thr * a * b, so the relative error is <= 16 eps_v / (thr * b) = 3.8e-6 * ext / (thr * b).
+//     Under thr * mn > 4e-3 * ext that is below 1e-3: within the slack.
+//   * Angle or band.  Edges at least ~0.6 degrees from parallel (|sin 2dT| > 0.02) have well-conditioned crossings.
+//     Near-parallel or near-perpendicular pairs must keep every pair of parallel edge lines more than RB_NMS_BAND * ext
+//     apart.  On (near-)parallel lines the reference's determinant is rounding noise of ~8 eps_v * L, and its t1, t2
+//     are gap * L over that noise: > 500 for a gap of 1e-3 * ext, so no false crossing point appears.  Lines that do
+//     cross inside the segments with a gap of 1e-3 * ext at the centre meet at an angle >= 2e-3 * ext / L, where the
+//     determinant is well conditioned again.  Boxes that share an edge line (same angle, same height, one nested in the
+//     other along the axis) are the failing case without this: the reference's clipper returns values up to 1.0 for a
+//     true IoU of 0.5, and such a pair must be clipped to reproduce them.
+// NaN or non-positive sizes fail the comparisons: no skip.
+#define RB_NMS_SLIVER 4e-3f
+#define RB_NMS_BAND 1e-3f
+RB_HD bool rbox_nms_cannot_exceed(const RBox& A, const RBox& B, float thr) {
+  if (!(thr > 0.0f && A.w > 0.0f && A.h > 0.0f && B.w > 0.0f && B.h > 0.0f)) return false;
+  const float dx = B.x - A.x, dy = B.y - A.y;
+  const float ext = fabsf(dx) + fabsf(dy) + A.r + B.r;
+  if (!(thr * fminf(A.mn, B.mn) > RB_NMS_SLIVER * ext)) return false;
+  const float sd = B.s2 * A.c2 - B.c2 * A.s2, cd = A.c2 * B.c2 + A.s2 * B.s2;
+  if (!(fabsf(sd * cd) > 0.000625f)) {                     // |sin 2dT| <= 0.02
+    const float S = 4.0f * fabsf(sd), C = 4.0f * fabsf(cd);
+    const float duA = 2.0f * (dx * A.c2 + dy * A.s2), dvA = 2.0f * (dy * A.c2 - dx * A.s2);
+    if (!rbox_parallel_edges_apart(A, B, duA, dvA, S, C, RB_NMS_BAND * ext)) return false;
+  }
+  const float ar = A.w * A.h, ac = B.w * B.h;
+  if (fminf(ar, ac) < 0.999f * thr * fmaxf(ar, ac)) return true;
+  const float ub = 1.001f * rbox_inter_upper_bound(A, B);
+  return ub < 0.999f * thr * (ar + ac - ub);
 }
 
 struct RPt { float x, y; };

@@ -56,4 +56,17 @@ void hh_inter_upper_bound(const float* b1, int64_t n, const float* b2, int64_t m
   }
 }
 
+// the NMS kernels' clip skip: 1 where the pair's IoU provably cannot exceed thr[i * m + j] (one threshold per pair)
+void hh_nms_cannot_exceed(const float* b1, int64_t n, const float* b2, int64_t m, const float* thr, uint8_t* out) {
+  for (int64_t i = 0; i < n; ++i) {
+    s2a::RBox A;
+    s2a::rbox_prep(b1[5*i], b1[5*i+1], b1[5*i+2], b1[5*i+3], b1[5*i+4], A);
+    for (int64_t j = 0; j < m; ++j) {
+      s2a::RBox B;
+      s2a::rbox_prep(b2[5*j], b2[5*j+1], b2[5*j+2], b2[5*j+3], b2[5*j+4], B);
+      out[i * m + j] = s2a::rbox_nms_cannot_exceed(A, B, thr[i * m + j]) ? 1 : 0;
+    }
+  }
+}
+
 }

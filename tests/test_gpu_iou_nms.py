@@ -5,13 +5,14 @@ CUDA kernels compiled for sm_100a and run on this box.
 
 Bars (BASELINE.json north_star): IoU within 1e-5 absolute of the reference (here: bit-exact
 against the oracle, i.e. against the reference header's device-side semantics without FMA
-contraction, except where the device's double-precision sin/cos differs from glibc's in the last
-bit -- such boxes are counted and bounded); NMS keep lists identical.
+contraction; only a box whose fp32 sin/cos may round differently on the device than in glibc
+(rbox_sets.angle_may_differ) is exempt, and no box of these sets is); NMS keep lists identical.
 """
 import numpy as np
 import pytest
 import torch
 
+import rbox_sets
 from conftest import bits
 from s2anet_b200 import synth
 
@@ -25,21 +26,22 @@ def gpu_iou(b1, b2, flags=0):
                            torch.from_numpy(np.ascontiguousarray(b2)).to(DEV), _flags=flags).cpu().numpy()
 
 
-def assert_iou_parity(mine, ref):
-    """bit-exact, tolerating only pairs that involve a box whose device sin/cos differs from libm."""
+def assert_iou_parity(mine, ref, b1, b2):
+    """Bit-exact.  The one allowed exception is a pair with a box whose float64 sin/cos lies so close to an fp32
+    rounding midpoint that CUDA's and glibc's (2 and 1 ulp accurate) may round it apart; such pairs must still be
+    within 1e-5.  None of the synthetic sets has such a box, so it is asserted that none is flagged."""
+    f1, f2 = rbox_sets.angle_may_differ(b1[:, 4]), rbox_sets.angle_may_differ(b2[:, 4])
+    assert not f1.any() and not f2.any(), "a synthetic box's sin/cos sits on an fp32 rounding midpoint"
     diff = bits(mine) != bits(ref)
-    assert np.abs(mine - ref).max() <= 1e-5, "IoU differs from the oracle by more than 1e-5"
-    frac = diff.mean()
-    assert frac <= 2e-3, "too many non-bit-exact pairs: %g" % frac
-    return frac
+    assert not diff.any(), "%d pairs differ from the oracle, first %s" % (diff.sum(), np.argwhere(diff)[:5].tolist())
 
 
 def test_iou_cfg1_golden_and_oracle(oracle, golden):
     g = golden("cfg1_iou_nms.npz")
     b = g["boxes"]
     mine = gpu_iou(b, b)
-    assert_iou_parity(mine[:200], g["iou_rows_0_200_ref_hdr_cuda"])
-    assert_iou_parity(mine, oracle.box_iou_rotated(b, b))
+    assert_iou_parity(mine[:200], g["iou_rows_0_200_ref_hdr_cuda"], b[:200], b)
+    assert_iou_parity(mine, oracle.box_iou_rotated(b, b), b, b)
     assert np.abs(mine[:200] - g["iou_rows_0_200_ref_ext_cpu"]).max() <= 1e-5     # reference CPU extension
     # the disjointness shortcut must not change a single bit
     np.testing.assert_array_equal(bits(mine), bits(gpu_iou(b, b, flags=1)))
@@ -57,7 +59,7 @@ def test_iou_adversarial_and_ragged(oracle, golden):
     for n, m in ((1, 1), (63, 65), (64, 64), (65, 1), (130, 257), (7, 500)):
         b1 = synth.clustered_boxes(n_seed=max(1, n), rep=1, seed=n)[0][:n]
         b2 = synth.clustered_boxes(n_seed=max(1, m // 2 + 1), rep=2, seed=m)[0][:m]
-        assert_iou_parity(gpu_iou(b1, b2), oracle.box_iou_rotated(b1, b2))
+        assert_iou_parity(gpu_iou(b1, b2), oracle.box_iou_rotated(b1, b2), b1, b2)
     assert gpu_iou(np.zeros((0, 5), np.float32), b2).shape == (0, len(b2))
     assert gpu_iou(b2, np.zeros((0, 5), np.float32)).shape == (len(b2), 0)
 
@@ -67,13 +69,13 @@ def test_iou_noncontiguous_input(oracle):
     b, s, _ = synth.clustered_boxes(n_seed=30, rep=3, seed=2)
     d6 = torch.from_numpy(np.concatenate([b, s[:, None]], 1)).to(DEV)
     out = bbox_iou_rotated(d6, d6[:, :5]).cpu().numpy()               # 6-column + strided view
-    assert_iou_parity(out, oracle.box_iou_rotated(b, b))
+    assert_iou_parity(out, oracle.box_iou_rotated(b, b), b, b)
 
 
 def test_iou_anchor_gt_golden_and_batched(oracle, golden):
     from s2anet_b200.box_iou_rotated import box_iou_rotated_batched
     g = golden("cfg4_anchor_gt_iou.npz")
-    assert_iou_parity(gpu_iou(g["anchors"], g["gts"]), g["iou_ref_hdr_cuda"])
+    assert_iou_parity(gpu_iou(g["anchors"], g["gts"]), g["iou_ref_hdr_cuda"], g["anchors"], g["gts"])
     # batched + row-sharded form equals per-image calls
     B = 3
     an = synth.all_level_anchors(B, 3)[:, ::8]
@@ -137,12 +139,12 @@ def test_iou_degenerate_pairs_take_the_general_clipper(oracle):
     triples: identical boxes, shared edges and corners, axis-aligned grid anchors against themselves) fall back to
     the general 24-point routine inside the same kernel: still bit-identical to the oracle."""
     ga = np.concatenate([synth.grid_anchors(16, 16, 8).reshape(-1, 5), synth.grid_anchors(8, 8, 16).reshape(-1, 5)])
-    assert_iou_parity(gpu_iou(ga, ga), oracle.box_iou_rotated(ga, ga))
+    assert_iou_parity(gpu_iou(ga, ga), oracle.box_iou_rotated(ga, ga), ga, ga)
     adv = synth.adversarial_boxes()
-    assert_iou_parity(gpu_iou(adv, ga[::3]), oracle.box_iou_rotated(adv, ga[::3]))
+    assert_iou_parity(gpu_iou(adv, ga[::3]), oracle.box_iou_rotated(adv, ga[::3]), adv, ga[::3])
     rot = ga.copy()
     rot[:, 4] = np.float32(np.pi / 4)
-    assert_iou_parity(gpu_iou(rot, ga), oracle.box_iou_rotated(rot, ga))
+    assert_iou_parity(gpu_iou(rot, ga), oracle.box_iou_rotated(rot, ga), rot, ga)
 
 
 def gpu_nms(b, s, thr, labels=None):

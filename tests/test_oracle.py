@@ -10,6 +10,7 @@ import subprocess
 import numpy as np
 import pytest
 
+import rbox_sets
 from conftest import ROOT, bits
 from s2anet_b200 import synth
 
@@ -158,6 +159,7 @@ def host_harness():
     f64p = np.ctypeslib.ndpointer(np.float64, flags="C")
     L.hh_poly_iou_pairs.argtypes = [f64p, f64p, C.c_int64, f64p]
     L.hh_inter_upper_bound.argtypes = [f32p, C.c_int64, f32p, C.c_int64, f32p]
+    L.hh_nms_cannot_exceed.argtypes = [f32p, C.c_int64, f32p, C.c_int64, f32p, np.ctypeslib.ndpointer(np.uint8, flags="C")]
 
     def run(b1, b2, mode):
         b1, b2 = np.ascontiguousarray(b1, np.float32), np.ascontiguousarray(b2, np.float32)
@@ -176,7 +178,13 @@ def host_harness():
         out_ = np.empty((len(b1), len(b2)), np.float32)
         L.hh_inter_upper_bound(b1, len(b1), b2, len(b2), out_)
         return out_
-    run.poly, run.bound = poly, bound
+    def skip(b1, b2, thr):
+        b1, b2 = np.ascontiguousarray(b1, np.float32), np.ascontiguousarray(b2, np.float32)
+        thr = np.ascontiguousarray(np.broadcast_to(np.asarray(thr, np.float32), (len(b1), len(b2))))
+        out_ = np.empty((len(b1), len(b2)), np.uint8)
+        L.hh_nms_cannot_exceed(b1, len(b1), b2, len(b2), thr, out_)
+        return out_.astype(bool)
+    run.poly, run.bound, run.skip = poly, bound, skip
     return run
 
 
@@ -195,15 +203,7 @@ def test_product_iou_source_on_host(oracle, host_harness):
     # slivers (sides down to 1e-4 of the pair distance and far beyond the guard) near and far from fat boxes, at
     # generic and at shared angles: the relaxed sliver guard (rbox_iou.cuh "Sliver guard") must still only ever
     # predict an exact zero where the reference computes one
-    rng = np.random.default_rng(11)
-    n = 400
-    thin = np.stack([rng.uniform(0, 2048, n), rng.uniform(0, 2048, n), 10 ** rng.uniform(0.5, 2.7, n),
-                     10 ** rng.uniform(-4, 0.7, n), rng.uniform(-np.pi / 4, 3 * np.pi / 4, n)], 1).astype(np.float32)
-    thin[::7, 4] = 0.0
-    thin[1::7, 4] = np.float32(np.pi / 2)
-    thin[2::7, 2:4] = thin[2::7, 3:1:-1]
-    fat = synth.dota_like_gt(300, 13)
-    fat[::5, 4] = 0.0
+    thin, fat = rbox_sets.thin_and_fat()
     sets.append((thin, fat))
     sets.append((thin, thin))
     for b1, b2 in sets:
@@ -242,3 +242,50 @@ def test_nms_intersection_bound_is_an_upper_bound(oracle, host_harness):
         assert not np.any(skipped & (iou > 0.5))
         if cand.sum() > 1000:
             assert (skipped & cand).sum() > 0.5 * cand.sum()
+
+
+def test_angle_screen():
+    """rbox_sets.angle_may_differ flags an angle whose float64 sine is 2 double ulps from an fp32 rounding midpoint
+    (found by a search over 10^8 random fp32 angles), not its neighbours, and almost no random angle."""
+    hit = np.array([0xbef3830f], np.uint32).view(np.float32)
+    assert rbox_sets.angle_may_differ(hit).all()
+    assert not rbox_sets.angle_may_differ(np.nextafter(hit, np.float32(1))).any()
+    t = np.random.default_rng(0).uniform(-np.pi, np.pi, 100000).astype(np.float32)
+    assert rbox_sets.angle_may_differ(t).sum() <= 2
+
+
+def test_nms_clip_skip_never_hides_a_suppression(oracle, host_harness):
+    """rbox_nms_cannot_exceed (the NMS kernels' "no clip" decision) may only say "cannot exceed thr" for a pair whose
+    oracle IoU is <= thr: at thr 0.1 ... 0.9 and just below each pair's own IoU (one ulp, 0.1 % and 1 % under).  The
+    sets hold what breaks a purely geometric bound: boxes sharing both long edge lines (the reference's IoU of such a
+    pair is up to 1.0 for a true 0.49), the same with the inner edges 1e-7 ... 1e-2 of the height apart, axis-aligned,
+    diagonal and vertical ones, slivers down to 1e-4 px, and the existing thin/fat, clustered and adversarial sets."""
+    sets = dict(rbox_sets.nested_sets())
+    sets["slivers"] = rbox_sets.slivers(300, 5)
+    thin, fat = rbox_sets.thin_and_fat()
+    sets["thin_fat"] = (thin, fat)
+    sets["thin_thin"] = thin
+    sets["clustered"] = synth.clustered_boxes(n_seed=150, rep=5, seed=5)[0]
+    sets["adversarial"] = synth.adversarial_boxes()
+    bad = {}
+    for name, s in sets.items():
+        b1, b2 = s if isinstance(s, tuple) else (s, s)
+        iou = oracle.box_iou_rotated(b1, b2)
+        with np.errstate(invalid="ignore"):
+            thrs = [np.float32(t) for t in (0.1, 0.3, 0.5, 0.7, 0.9)] + [
+                np.nextafter(iou, np.float32(-np.inf)), np.float32(0.999) * iou, np.float32(0.99) * iou]
+            for thr in thrs:
+                wrong = host_harness.skip(b1, b2, thr) & (iou > thr)
+                if wrong.any():
+                    bad[name] = bad.get(name, 0) + int(wrong.sum())
+    assert not bad, "pairs skipped although their IoU exceeds the threshold: %s" % bad
+    # the nested sets really are the hard case: many of their pairs sit far above the true IoU
+    g = sets["generic"]
+    v = np.array([oracle.single_iou(g[2 * k], g[2 * k + 1]) for k in range(len(g) // 2)])
+    assert (v > 0.5).sum() > 20
+    # and the skip is still useful: most overlapping-but-not-suppressing clustered pairs are decided without a clip
+    b = sets["clustered"]
+    iou = oracle.box_iou_rotated(b, b)
+    cand = (iou > 0) & (iou <= 0.5)
+    assert cand.sum() > 1000
+    assert (host_harness.skip(b, b, 0.5) & cand).sum() > 0.5 * cand.sum()

@@ -296,8 +296,8 @@ def sigmoid_in(x):
 
 
 def select_decode(cls_preds, bbox_preds, anchors, topk=2000, wh_ratio_clip=16 / 1000):
-    """models/head.py:684-717 for a batch: per level sigmoid, top-k by best class score (descending,
-    ties by ascending location), gather; concatenate levels; decode.  Returns (bboxes [B,n,5] fp32,
+    """models/head.py:684-717 for a batch: per level sigmoid, top-k by best class score (descending, NaN
+    first, ties by ascending location), gather; concatenate levels; decode.  Returns (bboxes [B,n,5] fp32,
     scores [B,n,C] fp32, index [B,n] int32)."""
     B = cls_preds[0].shape[0]
     out_b, out_s, out_i = [], [], []
@@ -310,8 +310,8 @@ def select_decode(cls_preds, bbox_preds, anchors, topk=2000, wh_ratio_clip=16 / 
             an = _f32(anc[b]).reshape(H * W, 5)
             idx = np.arange(H * W)
             if topk > 0 and H * W > topk:
-                best = sc.max(axis=1).astype(np.float32)
-                idx = np.lexsort((idx, -best))[:topk]
+                best = sc.max(axis=1).astype(np.float32)                # NaN if any class is NaN, like torch.max
+                idx = np.lexsort((idx, -best, ~np.isnan(best)))[:topk]  # NaN first, like torch.topk
             sl.append(sc[idx].astype(np.float32)); dl.append(de[idx]); al.append(an[idx]); il.append(idx.astype(np.int32))
         out_b.append(delta2bbox_rotated(np.concatenate(al), np.concatenate(dl), wh_ratio_clip))
         out_s.append(np.concatenate(sl)); out_i.append(np.concatenate(il))

@@ -56,6 +56,13 @@ __device__ __forceinline__ void load_channels(const T* q, long long cstride, lon
   }
 }
 
+// max that propagates NaN like torch.max (fmaxf drops it): a location with a NaN logit gets a NaN best score
+__device__ __forceinline__ float nan_max(float a, float b) { return (b > a || b != b) ? b : a; }
+
+// Top-k key of a best score: its bits (scores are >= 0, so they order like unsigned integers), NaN of either sign
+// mapped to the largest key -- the reference's topk ranks NaN above every number
+__device__ __forceinline__ uint32_t score_key(float s) { return s != s ? 0x7FFFFFFFu : __float_as_uint(s); }
+
 // torch.sigmoid on a T tensor: T(1 / (1 + exp(-float(x)))) (ATen UnarySpecialOpsKernel)
 template <typename T> __device__ __forceinline__ float sigmoid_t(float x) {
   return round_through<T>(__fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-x))));
@@ -135,7 +142,7 @@ __device__ __forceinline__ unsigned long long composite_key(uint32_t key, int i)
   return ((unsigned long long)key << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)i);
 }
 
-// Best class score of every location of one (level, image) -> keys[i] (bits of the T-rounded sigmoid), models/head.py:700-701.
+// Best class score of every location of one (level, image) -> keys[i] (score_key of the T-rounded sigmoid), models/head.py:700-701.
 // `t` of `NT` threads cooperate (a CTA, or the whole grid row of select_keys_kernel).
 template <typename T>
 __device__ __forceinline__ void compute_keys(const SelLevel& L, const T* cls, int C, int n, uint32_t* keys, int t, int NT) {
@@ -163,10 +170,10 @@ __device__ __forceinline__ void compute_keys(const SelLevel& L, const T* cls, in
         float m = -INFINITY;
 #pragma unroll
         for (int e = 0; e < 8; ++e)
-          if (half * 8 + e < C) m = fmaxf(m, bits16_to_float<T>((unsigned short)(w[e >> 1] >> ((e & 1) * 16))));
-        m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, 1));
+          if (half * 8 + e < C) m = nan_max(m, bits16_to_float<T>((unsigned short)(w[e >> 1] >> ((e & 1) * 16))));
+        m = nan_max(m, __shfl_xor_sync(0xffffffffu, m, 1));
         const int i = base + u * HALF_T + pr;
-        if (half == 0 && i < n) keys[i] = __float_as_uint(sigmoid_t<T>(m));
+        if (half == 0 && i < n) keys[i] = score_key(sigmoid_t<T>(m));
       }
     }
   } else
@@ -185,7 +192,7 @@ __device__ __forceinline__ void compute_keys(const SelLevel& L, const T* cls, in
         m[u] = -INFINITY;
 #pragma unroll
         for (int c = 0; c < 16; ++c)
-          if (c < C) m[u] = fmaxf(m[u], v[u][c]);
+          if (c < C) m[u] = nan_max(m[u], v[u][c]);
       }
     } else {
 #pragma unroll
@@ -194,14 +201,13 @@ __device__ __forceinline__ void compute_keys(const SelLevel& L, const T* cls, in
         const int y = i / L.W, x = i - y * L.W;
         const T* q = cls + y * L.cs[2] + x * L.cs[3];
         m[u] = -INFINITY;
-        for (int c = 0; c < C; ++c) m[u] = fmaxf(m[u], ld_as_float(q + c * L.cs[1]));
+        for (int c = 0; c < C; ++c) m[u] = nan_max(m[u], ld_as_float(q + c * L.cs[1]));
       }
     }
-    // sigmoid is monotone, so max_c sigmoid(x_c) == sigmoid(max_c x_c) bit for bit; scores are >= 0,
-    // so their bit patterns order like unsigned integers
+    // sigmoid is monotone, so max_c sigmoid(x_c) == sigmoid(max_c x_c) bit for bit
 #pragma unroll
     for (int u = 0; u < UNR; ++u)
-      if (i0 + u * NT < n) keys[i0 + u * NT] = __float_as_uint(sigmoid_t<T>(m[u]));
+      if (i0 + u * NT < n) keys[i0 + u * NT] = score_key(sigmoid_t<T>(m[u]));
   }
 }
 

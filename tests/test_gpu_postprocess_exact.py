@@ -13,8 +13,7 @@ Inputs cover the head's real layout (15 and 5 channels of 32-channel channels-la
 poisoned here so that any read past C changes the result), boundary tie groups larger than the part that is kept,
 fp16 subnormal and zero scores, +-0.0 scores, NaN scores and scores equal to the threshold.
 
-Known divergence, not tested: a NaN logit.  torch.max propagates it, so the reference ranks that location first;
-the kernel's fmaxf drops it and ranks the location by its other classes.
+Non-finite logits (NaN ranked first, as torch.max and torch.topk rank it) are tested in test_gpu_decode_exact.py.
 """
 import numpy as np
 import pytest
@@ -22,7 +21,7 @@ import torch
 
 from conftest import bits
 from s2anet_b200 import synth
-from test_decode import boxes_close
+from decode_reference import DeviceMath, assert_same
 
 DEV = "cuda:0"
 
@@ -33,12 +32,13 @@ DEV = "cuda:0"
 def reference_topk(scores, topk):
     """scores [n, C] of one (image, level), any float dtype -> the locations the per-level top-k keeps, in output
     order: all n in location order when topk <= 0 or n <= topk, else the topk best by max-over-classes score,
-    descending, equal scores by ascending location."""
+    descending, equal scores by ascending location.  As in the reference (torch.max, then torch.topk), a location with
+    a NaN class has a NaN best score, and NaN ranks above every number."""
     n = scores.shape[0]
     if topk <= 0 or n <= topk:
         return np.arange(n)
     best = np.asarray(scores, np.float64).max(axis=1)
-    return np.lexsort((np.arange(n), -best))[:topk]
+    return np.lexsort((np.arange(n), -best, ~np.isnan(best)))[:topk]
 
 
 def boundary_tie(scores, keep):
@@ -54,9 +54,10 @@ def _nhwc(x):
 
 
 def check_select_decode(cls, reg, anchors, topk):
-    """select_decode on the levels against reference_topk, with scores, gathers and boxes checked as well.
+    """select_decode on the levels against reference_topk, with scores and gathers checked as well, and the boxes bit
+    for bit against the decode model (tests/decode_reference.py).
     Returns [(image, level, n, k, tie group size, kept part of it)] for every level that selects."""
-    from s2anet_b200.decode import rboxes_decode_torch, select_decode
+    from s2anet_b200.decode import select_decode
     B, C = cls[0].shape[:2]
     fp32 = cls[0].dtype == torch.float32
     bb, sc, idx = select_decode(cls, reg, anchors, topk, return_index=True)
@@ -79,8 +80,10 @@ def check_select_decode(cls, reg, anchors, topk):
         assert torch.equal(ii, torch.from_numpy(want).to(DEV)), "level %d: top-k index differs" % l
         assert torch.equal(sc[:, off:off + k], ref_sc.gather(1, ii[..., None].expand(-1, -1, C)))
         assert torch.equal(bb[:, off:off + k], bb0[:, off0:off0 + n].gather(1, ii[..., None].expand(-1, -1, 5)))
-        want_b = rboxes_decode_torch(a.reshape(B, n, 5), _nhwc(r)).gather(1, ii[..., None].expand(-1, -1, 5))
-        assert boxes_close(bb[:, off:off + k].cpu().numpy(), want_b.cpu().numpy())
+        an, dl = a.reshape(B, n, 5).cpu().numpy(), _nhwc(r).float().cpu().numpy()
+        an, dl = np.stack([an[b][want[b]] for b in range(B)]), np.stack([dl[b][want[b]] for b in range(B)])
+        want_b = DeviceMath(DEV).decode(an, dl, c.dtype, 16 / 1000)
+        assert_same(bb[:, off:off + k].cpu().numpy(), want_b, "level %d: boxes differ from the decode model" % l)
         if n > k:
             for b in range(B):
                 ties.append((b, l, n, k) + boundary_tie(ref_np[b], want[b]))
@@ -193,7 +196,7 @@ def _place(vals, layout, dtype, poison):
         out = buf[:, 1:]
         out.copy_(v)
         assert out.data_ptr() % 16 != 0
-    assert torch.equal(out.float().cpu(), v.float())
+    assert_same(out.float().cpu().numpy(), v.float().numpy())           # (NaN == NaN)
     return out
 
 

@@ -111,6 +111,14 @@ S2A_EXPORT int s2a_nms_rotated(const float* dets, int64_t det_stride, const floa
  *   buffers (>= min(n*num_classes, max_per_img) to hold every possible result).
  * Sync-free and batched: `batch` images are processed by the same launches (image b reads
  * bboxes + b*n*5, scores + b*n*num_classes and writes row b of each output).
+ * Sizes: n < 2^30 and n <= 819,200 boxes per image (the per-class sweep holds 16 bytes per 64 boxes
+ * in shared memory, at most 200 KB), num_classes and batch <= 65535, and above 6,144 boxes per image
+ * batch*num_classes*n < 2^31 - 256; larger sizes return S2A_ERR_UNSUPPORTED.  iou_thr must be >= 0
+ * (S2A_ERR_UNSUPPORTED otherwise).
+ * workspace: s2a_multiclass_nms_rotated_workspace_bytes(n, num_classes, batch) bytes, dominated by the
+ * suppression mask of 8*batch*num_classes*n*ceil(n/64) bytes (for batch 8 and 15 classes: 0.68 GB
+ * at n = 6,720, 7.1 GB at n = 21,824); the rest is 48*batch*num_classes*n + 32*batch*n bytes, plus
+ * 16*batch*num_classes*n above 6,144 boxes per image (the sort keys).
  */
 S2A_EXPORT size_t s2a_multiclass_nms_rotated_workspace_bytes(int64_t n, int64_t num_classes,
                                                              int64_t batch);
@@ -125,7 +133,8 @@ S2A_EXPORT int s2a_multiclass_nms_rotated(const float* bboxes, const float* scor
  * count in column 0.  With ndests = 1 this is the "pack" of the NCCL all-gather done by the kernel that produces the
  * detections; with ndests = world the destinations are the ranks' symmetric buffers (this rank's own and its peers'
  * NVLink-mapped pointers, <= 8) and the stores ARE the all-gather -- the caller only adds a barrier
- * (s2anet_b200/dist.py, DetectionExchange).  Rows past the count are unspecified. */
+ * (s2anet_b200/dist.py, DetectionExchange).  Rows past the count are unspecified.  Size limits and workspace as for
+ * s2a_multiclass_nms_rotated. */
 S2A_EXPORT int s2a_multiclass_nms_rotated_packed(const float* bboxes, const float* scores, int64_t n,
                                                  int64_t num_classes, int64_t batch, float score_thr,
                                                  float iou_thr, int64_t max_per_img, float* const* dests,

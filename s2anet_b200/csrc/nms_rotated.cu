@@ -19,6 +19,8 @@
 // Results are identical to the reference CUDA semantics: predicate IoU > thr, IoU(earlier, later).
 #include <cub/cub.cuh>
 #include <float.h>
+#include <thrust/iterator/counting_iterator.h>
+#include <thrust/iterator/transform_iterator.h>
 
 #include "common.cuh"
 #include "rbox_iou.cuh"
@@ -393,7 +395,9 @@ static NmsWorkspace carve_nms(void* base, int64_t n) {
 // ------------------------------------------------------------------------------------------------
 constexpr int kSelThreads = 1024;
 constexpr int kSelItems = 6;                       // 1024 * 6 = 6144 boxes per image at most
-constexpr int kMcMaxBoxes = kSelThreads * kSelItems;
+constexpr int kMcMaxBoxes = kSelThreads * kSelItems;  // above it, the selection is a device-wide segmented sort
+constexpr int kMcSweepMaxSmem = 200 * 1024;               // the sweep's two bitmaps: 16 bytes per 64 boxes
+constexpr int kMcMaxSweepBoxes = kMcSweepMaxSmem / 16 * kBlk;   // 819,200 boxes per image
 
 __global__ void mc_prep_kernel(const float* __restrict__ bboxes, int64_t total, RBox* __restrict__ out) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -403,6 +407,19 @@ __global__ void mc_prep_kernel(const float* __restrict__ bboxes, int64_t total, 
     rbox_prep(d[0], d[1], d[2], d[3], d[4], b);
     out[i] = b;
   }
+}
+
+// Rank key of candidate box i: descending key order is descending score, equal scores in ascending box order.
+// Never 0 (the low word is >= 2^32 - 2^30), so 0 can pad a sort.
+__device__ __forceinline__ unsigned long long mc_rank_key(float sv, int i) {
+  // -0.0 and +0.0 are equal scores (ordered by box, like every other tie): one key for both
+  const unsigned u = sv == 0.0f ? 0u : __float_as_uint(sv);
+  const unsigned ord = (u & 0x80000000u) ? ~u : (u | 0x80000000u);       // unsigned order == float order
+  return ((unsigned long long)ord << 32) | (unsigned long long)(0xFFFFFFFFu - (unsigned)i);
+}
+
+__device__ __forceinline__ int mc_key_box(unsigned long long k) {
+  return (int)(0xFFFFFFFFu - (unsigned)(k & 0xFFFFFFFFull));
 }
 
 // One CTA per (class, image): ordered selection of the boxes whose class score exceeds the
@@ -430,10 +447,7 @@ __device__ __forceinline__ void mc_select_sort_body(const float* __restrict__ sc
     if (i < n) {
       const float sv = sc[(int64_t)i * C + c];
       if (sv > thr) {
-        // -0.0 and +0.0 are equal scores (ordered by box, like every other tie): one key for both
-        const unsigned u = sv == 0.0f ? 0u : __float_as_uint(sv);
-        const unsigned ord = (u & 0x80000000u) ? ~u : (u | 0x80000000u);       // unsigned order == float order
-        key[j] = ((unsigned long long)ord << 32) | (unsigned long long)(0xFFFFFFFFu - (unsigned)i);
+        key[j] = mc_rank_key(sv, i);
         ++local;
       }
     }
@@ -461,8 +475,7 @@ __device__ __forceinline__ void mc_select_sort_body(const float* __restrict__ sc
   }
   __syncthreads();
   for (int rank = threadIdx.x; rank < cnt; rank += kSelThreads) {
-    const unsigned long long k = s_keys[rank];
-    const int box = (int)(0xFFFFFFFFu - (unsigned)(k & 0xFFFFFFFFull));
+    const int box = mc_key_box(s_keys[rank]);
     seg_score[rank] = sc[(int64_t)box * C + c];           // (the input's bits: the key has no sign of zero)
     seg_box[rank] = box;
     seg_rbox[rank] = prepped[box];
@@ -481,6 +494,68 @@ mc_select_sort_kernel(const float* __restrict__ scores, int n, int C, float thr,
   mc_select_sort_body<ITEMS>(scores + (size_t)b * n * C, n, C, c, thr, prepped + (size_t)b * n,
                              seg_score + seg * n, seg_box + seg * n, seg_rbox + seg * n, seg_count + seg,
                              s_sort);
+}
+
+// Selection for n > kMcMaxBoxes, in three steps that produce what mc_select_sort_body produces:
+//   mc_key_kernel      one thread per (image, box, class) score: the candidate's rank key is appended to its segment's
+//                      slice [seg * n, seg * n + n) of `keys` (warp-aggregated atomics on seg_count, which must be
+//                      zero on entry).  The append order varies from run to run; the keys of a segment are unique,
+//                      so their sorted order does not.
+//   cub::DeviceSegmentedRadixSort, descending, over [seg * n, seg * n + seg_count[seg]) (end offsets read on the
+//                      device: no host round trip).
+//   mc_gather_kernel   one thread per (segment, rank < count): the input's score bits, the box, the prepared box.
+__global__ void mc_key_kernel(const float* __restrict__ scores, int n, int C, float thr,
+                              unsigned long long* __restrict__ keys, int* __restrict__ seg_count) {
+  const int b = blockIdx.y;
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;       // < n * C (< 2^31, checked by the host)
+  const int i = e / C, c = e - i * C;
+  const bool in = e < n * C;
+  const float sv = in ? scores[((size_t)b * n + i) * C + c] : 0.0f;
+  const bool cand = in && sv > thr;
+  const unsigned cm = __ballot_sync(0xffffffffu, cand);
+  if (!cand) return;
+  const int seg = b * C + c;
+  const unsigned peers = __match_any_sync(cm, seg);
+  const int lane = threadIdx.x & 31, leader = __ffs(peers) - 1;
+  int base = 0;
+  if (lane == leader) base = atomicAdd(&seg_count[seg], __popc(peers));
+  base = __shfl_sync(peers, base, leader);
+  keys[(size_t)seg * n + base + __popc(peers & ((1u << lane) - 1u))] = mc_rank_key(sv, i);
+}
+
+__global__ void mc_gather_kernel(const float* __restrict__ scores, int n, int C,
+                                 const unsigned long long* __restrict__ keys, const int* __restrict__ seg_count,
+                                 const RBox* __restrict__ prepped, float* __restrict__ seg_score,
+                                 int* __restrict__ seg_box, RBox* __restrict__ seg_rbox) {
+  const int c = blockIdx.y, b = blockIdx.z;
+  const size_t seg = (size_t)b * C + c;
+  const int rank = blockIdx.x * blockDim.x + threadIdx.x;
+  if (rank >= seg_count[seg]) return;
+  const size_t o = seg * n + rank;
+  const int box = mc_key_box(keys[o]);
+  seg_score[o] = scores[((size_t)b * n + box) * C + c];     // (the input's bits: the key has no sign of zero)
+  seg_box[o] = box;
+  seg_rbox[o] = prepped[(size_t)b * n + box];
+}
+
+struct McSegBegin {
+  int n;
+  __host__ __device__ int operator()(int s) const { return s * n; }
+};
+struct McSegEnd {
+  int n;
+  const int* count;
+  __host__ __device__ int operator()(int s) const { return s * n + count[s]; }
+};
+using McBeginIt = thrust::transform_iterator<McSegBegin, thrust::counting_iterator<int>>;
+using McEndIt = thrust::transform_iterator<McSegEnd, thrust::counting_iterator<int>>;
+
+static cudaError_t mc_segmented_sort(void* tmp, size_t& tmp_bytes, cub::DoubleBuffer<unsigned long long>& keys, int n,
+                                     int S, const int* seg_count, cudaStream_t st) {
+  const thrust::counting_iterator<int> s0(0);
+  return cub::DeviceSegmentedRadixSort::SortKeysDescending(tmp, tmp_bytes, keys, S * n, S,
+                                                           McBeginIt(s0, McSegBegin{n}),
+                                                           McEndIt(s0, McSegEnd{n, seg_count}), 0, 64, st);
 }
 
 // exclusive prefix of the per-segment tile counts (upper triangle incl. diagonal)
@@ -630,9 +705,13 @@ __global__ void mc_emit_kernel(const float* __restrict__ bboxes, const float* __
 
 struct McWorkspace {
   RBox* prepped; float* seg_score; int* seg_box; RBox* seg_rbox; int* seg_count; long long* tile_off;
-  unsigned long long* mask; float* kept_score; int* kept_box; int* kept_count; size_t total;
+  unsigned long long* mask; float* kept_score; int* kept_box; int* kept_count;
+  unsigned long long* keys[2]; void* sort_tmp; size_t sort_bytes;       // n > kMcMaxBoxes only
+  size_t total;
 };
 
+// The mask, [B * C][n][ceil(n / 64)] words, dominates: for B = 8 and C = 15, 0.68 GB at n = 6,720 and 7.1 GB at
+// n = 21,824.  Above kMcMaxBoxes two [B * C][n] key buffers and the segmented sort's scratch are added.
 static McWorkspace carve_mc(void* base, int64_t n, int64_t C, int64_t B) {
   McWorkspace w;
   const int64_t S = B * C, ld = ceil_div(n, kBlk);
@@ -648,6 +727,16 @@ static McWorkspace carve_mc(void* base, int64_t n, int64_t C, int64_t B) {
   w.kept_score = (float*)take(sizeof(float) * S * n);
   w.kept_box = (int*)take(sizeof(int) * S * n);
   w.kept_count = (int*)take(sizeof(int) * S);
+  w.keys[0] = w.keys[1] = nullptr;
+  w.sort_tmp = nullptr;
+  w.sort_bytes = 0;
+  if (n > kMcMaxBoxes && S * n < (1ll << 31) - 256) {           // (larger S * n is refused by multiclass_impl)
+    w.keys[0] = (unsigned long long*)take(sizeof(unsigned long long) * S * n);
+    w.keys[1] = (unsigned long long*)take(sizeof(unsigned long long) * S * n);
+    cub::DoubleBuffer<unsigned long long> db(nullptr, nullptr);
+    mc_segmented_sort(nullptr, w.sort_bytes, db, (int)n, (int)S, nullptr, 0);
+    w.sort_tmp = take(w.sort_bytes);
+  }
   w.total = off;
   return w;
 }
@@ -786,16 +875,24 @@ static int multiclass_impl(const float* bboxes, const float* scores, int64_t n, 
   }
   S2A_CHECK_ARG(bboxes && scores && workspace, "multiclass_nms_rotated: null pointer");
   S2A_CHECK_ARG(max_out > 0, "multiclass_nms_rotated: max_out must be positive");
-  if (n > kMcMaxBoxes) {
-    set_error("multiclass_nms_rotated: fused path supports n <= %d boxes per image (got %lld); "
-              "compose s2a_nms_rotated instead", kMcMaxBoxes, (long long)n);
-    return S2A_ERR_UNSUPPORTED;
-  }
+  S2A_CHECK_ARG(n < (1ll << 30), "multiclass_nms_rotated: n (%lld) out of range", (long long)n);
   if (!(iou_thr >= 0.0f)) {
     set_error("multiclass_nms_rotated: class-segmented path needs iou_thr >= 0 (got %g)", (double)iou_thr);
     return S2A_ERR_UNSUPPORTED;
   }
   S2A_CHECK_ARG(num_classes <= 65535 && batch <= 65535, "multiclass_nms_rotated: classes/batch must be <= 65535");
+  // the per-segment sweep keeps two bitmaps of ceil(n / 64) words in shared memory
+  const size_t smem = 2 * sizeof(unsigned long long) * (size_t)ceil_div(n, kBlk);
+  if (smem > kMcSweepMaxSmem) {
+    set_error("multiclass_nms_rotated: n (%lld) above %d boxes per image, the most the per-class sweep holds in "
+              "shared memory", (long long)n, kMcMaxSweepBoxes);
+    return S2A_ERR_UNSUPPORTED;
+  }
+  if (n > kMcMaxBoxes && batch * num_classes * n >= (1ll << 31) - 256) {
+    set_error("multiclass_nms_rotated: batch * classes * n (%lld) must be below 2^31 - 256 above %d boxes per image",
+              (long long)(batch * num_classes * n), kMcMaxBoxes);
+    return S2A_ERR_UNSUPPORTED;
+  }
   McWorkspace w = carve_mc(workspace, n, num_classes, batch);
   if (workspace_bytes < w.total) {
     set_error("multiclass_nms_rotated: workspace too small (%zu < %zu bytes)", workspace_bytes, w.total);
@@ -805,12 +902,26 @@ static int multiclass_impl(const float* bboxes, const float* scores, int64_t n, 
   const int ld = (int)ceil_div(n, kBlk);
   mc_prep_kernel<<<(unsigned)ceil_div(batch * n, 256), 256, 0, st>>>(bboxes, batch * n, w.prepped);
   S2A_LAUNCH_OK("mc_prep_kernel");
-  dim3 gsel(C, B);
-  cudaError_t e;
-  if (ni <= kSelThreads) e = launch_select_sort<1>(gsel, st, scores, ni, C, score_thr, w);
-  else if (ni <= 2 * kSelThreads) e = launch_select_sort<2>(gsel, st, scores, ni, C, score_thr, w);
-  else e = launch_select_sort<kSelItems>(gsel, st, scores, ni, C, score_thr, w);
-  S2A_CUDA_OK(e);
+  if (ni <= kMcMaxBoxes) {
+    dim3 gsel(C, B);
+    cudaError_t e;
+    if (ni <= kSelThreads) e = launch_select_sort<1>(gsel, st, scores, ni, C, score_thr, w);
+    else if (ni <= 2 * kSelThreads) e = launch_select_sort<2>(gsel, st, scores, ni, C, score_thr, w);
+    else e = launch_select_sort<kSelItems>(gsel, st, scores, ni, C, score_thr, w);
+    S2A_CUDA_OK(e);
+  } else {
+    S2A_CUDA_OK(cudaMemsetAsync(w.seg_count, 0, sizeof(int) * S, st));
+    mc_key_kernel<<<dim3((unsigned)ceil_div(n * C, 256), B), 256, 0, st>>>(scores, ni, C, score_thr, w.keys[0],
+                                                                           w.seg_count);
+    S2A_LAUNCH_OK("mc_key_kernel");
+    cub::DoubleBuffer<unsigned long long> db(w.keys[0], w.keys[1]);
+    size_t sort_bytes = w.sort_bytes;
+    S2A_CUDA_OK(mc_segmented_sort(w.sort_tmp, sort_bytes, db, ni, S, w.seg_count, st));
+    mc_gather_kernel<<<dim3((unsigned)ceil_div(n, 256), C, B), 256, 0, st>>>(scores, ni, C, db.Current(), w.seg_count,
+                                                                             w.prepped, w.seg_score, w.seg_box,
+                                                                             w.seg_rbox);
+    S2A_LAUNCH_OK("mc_gather_kernel");
+  }
   // (thread 0 walks the per-thread partial sums serially: no more threads than segments)
   const int scan_threads = (int)std::min<int64_t>(1024, align_up((size_t)S, 32));
   mc_tile_scan_kernel<<<1, scan_threads, 0, st>>>(w.seg_count, S, w.tile_off);
@@ -818,7 +929,8 @@ static int multiclass_impl(const float* bboxes, const float* scores, int64_t n, 
   mc_mask_kernel<<<sm_count() * 5, kTileThreads, 0, st>>>(w.seg_rbox, w.seg_count, w.tile_off, S, ni, ld, iou_thr,
                                                           w.mask);
   S2A_LAUNCH_OK("mc_mask_kernel");
-  const size_t smem = 2 * sizeof(unsigned long long) * (size_t)ld;
+  if (smem > 48 * 1024)
+    S2A_CUDA_OK(cudaFuncSetAttribute(mc_sweep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   mc_sweep_kernel<<<S, kSweepThreads, smem, st>>>(w.mask, w.seg_count, ni, ld, w.seg_score, w.seg_box,
                                                   w.kept_score, w.kept_box, w.kept_count);
   S2A_LAUNCH_OK("mc_sweep_kernel");

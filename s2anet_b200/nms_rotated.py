@@ -61,13 +61,16 @@ def nms_rotated(dets, iou_thr):
     return dets, keep_inds
 
 
-MC_FUSED_MAX_BOXES = 6144      # kMcMaxBoxes in csrc/nms_rotated.cu
+# kMcMaxBoxes in csrc/nms_rotated.cu: the most boxes per image whose per-class selection runs in one CTA.  The fused
+# path takes any n; above this it selects with a device-wide segmented sort instead.
+MC_FUSED_MAX_BOXES = 6144
 
 
 def multiclass_nms_rotated_batched(bboxes, scores, score_thr=0.05, iou_thr=0.5, max_per_img=2000):
     """Fused, sync-free, batched form: bboxes [B,n,5], scores [B,n,C] ->
     (dets [B,max_per_img,6], labels [B,max_per_img] float32, counts [B] int32); rows >= counts[b]
-    are unspecified.  One call = 6 kernel launches for the whole batch, no host round trip."""
+    are unspecified.  No host round trip at any n: one call = 6 kernel launches for the whole batch up to
+    MC_FUSED_MAX_BOXES boxes per image, plus the segmented sort's passes above it."""
     dev = _lib.require_cuda(bboxes, scores)
     B, n, _ = bboxes.shape
     C = scores.size(2)
@@ -79,10 +82,9 @@ def multiclass_nms_rotated_batched(bboxes, scores, score_thr=0.05, iou_thr=0.5, 
     counts = torch.zeros((B,), dtype=torch.int32, device=dev)
     if B == 0 or n == 0 or C == 0:
         return dets, labels, counts
-    if n > MC_FUSED_MAX_BOXES or not (iou_thr >= 0):
-        # Sizes the fused kernel does not take (more than 6,144 candidate boxes per image -- e.g. 5 levels x top-2000
-        # on inputs above ~1,100 px -- or a negative threshold): per image, the reference's own composition on the
-        # generic ml_nms_rotated kernel (one 4-byte host read per image), written into the same fixed-shape outputs.
+    if not (iou_thr >= 0):
+        # A negative threshold, which the fused kernel does not take: per image, the reference's own composition on
+        # the generic ml_nms_rotated kernel (one 4-byte host read per image), written into the same fixed-shape outputs.
         for b in range(B):
             d, l = _multiclass_composed(bboxes[b], scores[b], score_thr, iou_thr, max_per_img)
             k = d.size(0)
@@ -100,6 +102,8 @@ def multiclass_nms_rotated_batched(bboxes, scores, score_thr=0.05, iou_thr=0.5, 
                                             _lib.ptr(counts), max_out, _lib.ptr(ws), ws_bytes,
                                             _lib.stream_ptr(dev))
     _lib.check(rc, "multiclass_nms_rotated")
+    if n > MC_FUSED_MAX_BOXES:
+        _lib.launches += 1        # (a key and a gather kernel in place of the select kernel)
     return dets, labels, counts
 
 
@@ -107,16 +111,16 @@ def multiclass_nms_rotated_packed(bboxes, scores, dests, slot0=0, score_thr=0.05
     """The batched NMS writing PACKED rows into one or several [slots, K+1, 8] buffers (see
     s2a_multiclass_nms_rotated_packed): `dests` is a list of fp32 tensors and / or raw device pointers (ints: the
     NVLink-mapped buffers of peer ranks, dist.DetectionExchange.targets()); image b lands in slot slot0 + b.
-    K (rows per image) defaults to dests[0].size(1) - 1.  Sync-free, graph-capturable, 6 launches."""
+    K (rows per image) defaults to dests[0].size(1) - 1.  Sync-free and graph-capturable at any n."""
     import ctypes as C
     dev = _lib.require_cuda(bboxes, scores)
     B, n, _ = bboxes.shape
     nc = scores.size(2)
     if K is None:
         K = dests[0].size(1) - 1
-    if n > MC_FUSED_MAX_BOXES or not (iou_thr >= 0):
-        raise NotImplementedError("multiclass_nms_rotated_packed: the fused path takes n <= %d boxes and iou_thr >= 0; "
-                                  "use multiclass_nms_rotated_batched + dist.gather_detections" % MC_FUSED_MAX_BOXES)
+    if not (iou_thr >= 0):
+        raise NotImplementedError("multiclass_nms_rotated_packed: the fused path takes iou_thr >= 0; "
+                                  "use multiclass_nms_rotated_batched + dist.gather_detections")
     bboxes = bboxes.to(torch.float32).contiguous()
     scores = scores.to(torch.float32).contiguous()
     ptrs = (C.c_void_p * len(dests))(*[d.data_ptr() if torch.is_tensor(d) else int(d) for d in dests])
@@ -128,10 +132,12 @@ def multiclass_nms_rotated_packed(bboxes, scores, dests, slot0=0, score_thr=0.05
                                                    float(iou_thr), int(max_per_img), ptrs, len(dests), int(slot0), int(K),
                                                    _lib.ptr(ws), ws_bytes, _lib.stream_ptr(dev))
     _lib.check(rc, "multiclass_nms_rotated_packed")
+    if n > MC_FUSED_MAX_BOXES:
+        _lib.launches += 1        # (a key and a gather kernel in place of the select kernel)
 
 
 def _multiclass_composed(bboxes, scores, score_thr, iou_thr, max_per_img):
-    """Sizes the fused kernel does not take (n > 6144 boxes, negative thresholds): the reference's
+    """Negative thresholds, which the fused kernel does not take, and the tests' witness for it: the reference's
     own composition (utils/bbox_nms_rotated.py:24-64) on top of the generic ml_nms_rotated kernel."""
     num_classes = scores.size(1)
     boxes = bboxes[:, None].expand(-1, num_classes, 5)
@@ -153,7 +159,7 @@ def multiclass_nms_rotated(bboxes, scores, score_thr=0.05, iou_thr=0.5, max_per_
     (dets [k,6], labels [k]); labels are float like the reference's `labels.to(bboxes)`, and the
     empty case returns ([0,6], [0,1] int64) like the reference's else-branch (:60-64)."""
     assert bboxes.shape[1] == 5
-    if bboxes.size(0) > MC_FUSED_MAX_BOXES or not (iou_thr >= 0):
+    if not (iou_thr >= 0):
         return _multiclass_composed(bboxes, scores, score_thr, iou_thr, max_per_img)
     dets, labels, counts = multiclass_nms_rotated_batched(bboxes[None], scores[None], score_thr, iou_thr,
                                                           max_per_img)
